@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Throughput benchmark of the association hot path (driver contract: one JSON line on stdout).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--config cfg2|cfg3|cfg4|cfg5]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--config cfg2|cfg3|cfg4|cfg5] [--dump-outputs DIR]
     torchrun --nnodes=1 --nproc-per-node N ... bench.py --gpus N --steps K --warmup W
 
 Default workload = BASELINE.json configs[3] / SURVEY §8d cfg4, the configuration the metric is quoted on:
@@ -21,7 +21,11 @@ roofline: dominant kernel = the TMA-fed tcgen05 3x3-conv contraction of the VGG 
 kernels : the same per-launch timing for EVERY hot kernel of the path, tagged (stage, layer): algorithmic FLOPs and
           compulsory HBM bytes of the launch / its measured duration, against the measured tensor / HBM peak.
 cpu_baseline / --impl reference: the oracle port of the reference's PyTorch-CPU path (the reference is pure Python and
-          /root/reference does not exist on the GPU box) on the host cores (thread count swept on the real shape).
+          is not needed at run time) on the host cores (thread count swept on the real shape); --impl reference times one
+          frame-pair per step, --steps of them.
+--dump-outputs DIR: after the timed steps, every array the timed path returned in its last step, as DIR/<name>.npy
+          (float32, or float64 for integer outputs; cfg5: per sweep point, prefixed n<N>_).  Inputs and weights are
+          seeded, so two builds run with the same arguments can be compared output for output.
 """
 import argparse
 import ctypes
@@ -168,7 +172,8 @@ def pick_cpu_threads(c):
 
 def oracle_pairs_per_s(c, n_pairs, threads, budget_s=60.0):
     """The reference's CPU path (oracle port of TrackingNet.forward + HiGHS restatement of the LP; cfg5: associate +
-    LP only).  Bounded sample: stops early once `budget_s` seconds of CPU work are spent (>= 1 pair is always timed)."""
+    LP only).  Bounded sample: stops early once `budget_s` seconds of CPU work are spent (>= 1 pair is always timed;
+    budget_s=None times all n_pairs)."""
     from mmmot_b200.synthetic import synthetic_pair, synthetic_state_dict
     from oracle import lp_ref, torch_ref
     torch.set_num_threads(threads)
@@ -191,15 +196,15 @@ def oracle_pairs_per_s(c, n_pairs, threads, budget_s=60.0):
             z = torch.zeros(n)
             lp_ref.milp_solve(det, [link[2]], torch.cat([z, new[2]]), torch.cat([end[2], z]), [n, n])
         t_tot += time.perf_counter() - t
-        if t_tot > budget_s:
+        if budget_s is not None and t_tot > budget_s:
             n_pairs = p + 1
             break
     return n_pairs / t_tot, t_tot, n_pairs
 
 
-def cpu_leg(c, n_pairs):
+def cpu_leg(c, n_pairs, budget_s=60.0):
     threads, sweep = pick_cpu_threads(c)
-    rate, secs, done = oracle_pairs_per_s(c, n_pairs, threads)
+    rate, secs, done = oracle_pairs_per_s(c, n_pairs, threads, budget_s)
     what = "forward + LP" if c["hw"] else "affinity stage + LP"
     return {"value": rate, "unit": "frame-pairs/s", "cores": threads, "host_cores": os.cpu_count(), "kind": "port",
             "thread_sweep_s": sweep,
@@ -216,10 +221,43 @@ def config_dict(c, name, pairs, world, scaling):
     return d
 
 
+DUMP_LIMIT = 64 << 20          # bytes written by --dump-outputs, all arrays together
+
+
+def _dump_bytes(t):
+    return t.numel() * (4 if t.dtype == torch.float32 else 8)
+
+
+def dump_outputs(out_dir, sets):
+    """--dump-outputs: every output of the last timed step as <out_dir>/<name>.npy, float32 as computed and every other
+    dtype (int32 indices, the status word) as float64, which holds it exactly.  `sets` is a list of
+    (prefix, per_pair, shared, B): per_pair maps names (prefix included) to tensors whose leading axis is the B
+    frame-pairs, shared to tensors without one.  When the whole would exceed DUMP_LIMIT, every per-pair array keeps the
+    same fixed, seeded subset of its frame-pairs, and the indices kept are written as <prefix>pair_index.npy."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    limit = DUMP_LIMIT - (1 << 20)                       # headroom for the .npy headers
+    total = sum(_dump_bytes(t) for _, pp, sh, _ in sets for t in list(pp.values()) + list(sh.values()))
+    shared = sum(_dump_bytes(t) for _, _, sh, _ in sets for t in sh.values())
+    index = 8 * sum(B for _, _, _, B in sets)            # the pair_index arrays, when sampling
+    frac = 1.0 if total <= limit else (limit - shared) / (total - shared + index)
+    for prefix, per_pair, sh, B in sets:
+        arrays = dict(sh)
+        if frac < 1.0:
+            keep = torch.randperm(B, generator=torch.Generator().manual_seed(0))[:max(1, int(B * frac))].sort().values
+            arrays[prefix + "pair_index"] = keep
+            arrays.update({k: v[keep.to(v.device)] for k, v in per_pair.items()})
+        else:
+            arrays.update(per_pair)
+        for k, v in arrays.items():
+            v = v.detach().cpu()
+            np.save(os.path.join(out_dir, k + ".npy"), (v if v.dtype == torch.float32 else v.double()).numpy())
+
+
 def run_reference(args, c, name, rank):
     if rank != 0:
         return
-    cpu, secs, done = cpu_leg(c, max(args.steps, 1))
+    cpu, secs, done = cpu_leg(c, args.steps, budget_s=None)       # one frame-pair per step, every step timed
     line = {"impl": "reference", "metric": metric_name(c), "value": cpu["value"], "unit": "frame-pairs/s", "n_gpus": args.gpus,
             "steps": args.steps, "warmup": args.warmup, "ms_per_step": 1e3 * secs / max(done, 1),
             "higher_is_better": True, "scaling": "weak", "vs_baseline": None, "dtype": "f32", "data": "synthetic",
@@ -287,7 +325,7 @@ def run_sweep(args, c, name, rank, world, local):
     peaks, how = load_peaks()
     sampler = ClockSampler(local)
     sampler.start()
-    points, main = [], None
+    points, main, dumps = [], None, []
     for n in SWEEP_N:
         # batch sized so that one step is >= ~100 ms of device work and inputs exceed L2 where they can
         B = args.pairs if args.pairs else max(16, min(4096, int(32 * (128 / n) ** 2)))
@@ -299,9 +337,13 @@ def run_sweep(args, c, name, rank, world, local):
         d_feats = torch.empty_like(feats)
         zn = torch.zeros(B, n, device=dev)
 
+        last = {}
+
         def step(f):
             link, new, end = net.associate_batch(f, n)
-            return mmmot_b200.solve_batch(det, link[:, 2], torch.cat([zn, new[:, 2]], 1), torch.cat([end[:, 2], zn], 1), n, n)
+            r = mmmot_b200.solve_batch(det, link[:, 2], torch.cat([zn, new[:, 2]], 1), torch.cat([end[:, 2], zn], 1), n, n)
+            last.update(r, link=link, new=new, end=end)
+            return r
 
         def step_e2e():
             d_feats.copy_(h_feats, non_blocking=True)
@@ -324,6 +366,8 @@ def run_sweep(args, c, name, rank, world, local):
             lib.mmmot_timing_enable(0)
             return e0.elapsed_time(e1), lib.mmmot_launch_count() - l0, (collect_tags(lib) if hooks else None)
         ms, launches, tags = timed(lambda: step(feats), True)
+        if args.dump_outputs:
+            dumps.append((f"n{n}_", {f"n{n}_{k}": v for k, v in last.items()}, {}, B))
         ms2, _, _ = timed(step_e2e, False)
         pt = {"n": n, "pairs_per_step": B, "value": B * args.steps / (ms / 1e3), "e2e": B * args.steps / (ms2 / 1e3),
               "ms_per_step": ms / args.steps, "gpu_launches": int(launches),
@@ -350,6 +394,8 @@ def run_sweep(args, c, name, rank, world, local):
                          "achieved": l1["algorithmic_tflops"], "peak": peaks.get("bf16_tflops_sustained", 1400.0), "unit": "TFLOP/s",
                          "frac": l1["frac"], "peak_source": f"{how} bf16_tflops_sustained", "traffic": None},
             "kernels": pt["kernels"], "sweep": points, "cpu_baseline": cpu}
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, dumps)
     print(json.dumps(line), flush=True)
 
 
@@ -369,7 +415,15 @@ def main():
     ap.add_argument("--kseg", type=int, default=-1, help="tcgen05 conv K-segment length in 32-chunks (0 = off; default: library default)")
     ap.add_argument("--engine", default="auto", choices=["auto", "fp32", "tcgen05"],
                     help="contraction engine (A/B runs; default auto = tcgen05 for this workload)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last timed step computed as DIR/<name>.npy (rank 0; at most "
+                         "64 MB in all, a fixed seeded sample of the frame-pairs beyond that); the inputs are seeded, so two "
+                         "builds can be compared output for output")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be >= 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the CUDA path's outputs; the reference arm has none")
     rank = int(os.environ.get("RANK", 0))
     world = int(os.environ.get("WORLD_SIZE", 1))
     local = int(os.environ.get("LOCAL_RANK", 0))
@@ -447,6 +501,7 @@ def main():
         else:
             last["match"] = o["match"]
         last["status"] = o["status"]
+        last["out"] = o
         return o
 
     # e2e = the package's own host pipeline (mmmot_b200.HostPipeline): pinned host -> device copies overlapped with
@@ -566,6 +621,14 @@ def main():
         if world > 1:
             line["shard_equal"] = shard_equal
         assert status == 0, "MMMOT_E_RANGE raised during the benchmark"
+        if args.dump_outputs:
+            o = last["out"]
+            per_pair = {k: o[k] for k in ("det", "link", "new", "end", "assign_det", "assign_link", "assign_new",
+                                          "assign_end", "match")}
+            sets = [("", per_pair, {"trans1": o["trans"][0], "trans2": o["trans"][1], "status": o["status"]}, B)]
+            if world > 1:        # what the final gather hands rank 0: every rank's assignment indices
+                sets.append(("gathered_", {"gathered_match": last["match"]}, {}, total))
+            dump_outputs(args.dump_outputs, sets)
         print(json.dumps(line), flush=True)
     if world > 1:
         dist.destroy_process_group()

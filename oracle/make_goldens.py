@@ -48,6 +48,20 @@ def reference_forward(case, want_feats=False):
             "trans1": trans[0], "trans2": trans[1], "feats": feats}
 
 
+# BASELINE config[0]: the Fusion-A N=8 plumbing case at 64x64 crops
+LIVE_CASE = ("cfg1_mul_A_n8", "A", "multiply", "none", 0.2, 8, 8, 64, 64, False, 21)
+
+
+def live_golden():
+    """The reference's eval-mode outputs of LIVE_CASE (det, link, new, end), stored as float32 arrays so that
+    tests/test_oracle.py checks the oracle against them without the reference tree."""
+    import numpy as np
+    ref = reference_forward(LIVE_CASE)
+    np.savez_compressed(os.path.join(OUT, LIVE_CASE[0] + ".npz"),
+                        **{k: ref[k].numpy().astype(np.float32) for k in ("det", "link", "new", "end")})
+    print(LIVE_CASE[0], {k: tuple(ref[k].shape) for k in ("det", "link", "new", "end")})
+
+
 def crop_goldens():
     """LiDAR cropping (SURVEY §8f N1) through the UNMODIFIED reference functions (numba):
     box_np_ops.box_camera_to_lidar + preprocess.remove_points_outside_boxes, per box, empty box -> zero point."""
@@ -249,6 +263,7 @@ def main():
     crop_goldens()
     resize_goldens()
     stitch_goldens()
+    live_golden()
     torch.set_num_threads(os.cpu_count())
     for case in CASES:
         out = reference_forward(case)

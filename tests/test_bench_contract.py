@@ -60,3 +60,49 @@ def test_reference_arm_prints_a_contract_line_without_a_gpu():
     assert d["impl"] == "reference" and d["gpu_launches"] == 0 and d["value"] > 0
     assert d["cpu_baseline"]["value"] == d["value"] and d["e2e"]["value"] == d["value"]
     assert d["e2e"]["h2d_bytes_per_step"] == 0 and d["e2e"]["d2h_bytes_per_step"] == 0
+
+
+def test_dump_outputs_keeps_a_fixed_sample_under_the_limit(tmp_path):
+    """bench.dump_outputs writes float32 as computed and integer outputs as float64; past DUMP_LIMIT every per-pair array
+    keeps the same seeded subset of frame-pairs, recorded in pair_index.npy, and the files stay under the limit."""
+    import numpy as np
+    import torch
+    import bench
+    B = 256
+    g = torch.Generator().manual_seed(0)
+    per_pair = {"link": torch.rand(B, 3, 128, 128, generator=g), "match": torch.randint(-1, 128, (B, 128), generator=g, dtype=torch.int32)}
+    shared = {"trans2": torch.rand(1, 64, 64, generator=g), "status": torch.zeros(1, dtype=torch.int32)}
+    bench.dump_outputs(str(tmp_path / "a"), [("", per_pair, shared, B)])
+    bench.dump_outputs(str(tmp_path / "b"), [("", per_pair, shared, B)])
+    a = {f: np.load(tmp_path / "a" / f) for f in os.listdir(tmp_path / "a")}
+    assert set(a) == {"link.npy", "match.npy", "trans2.npy", "status.npy"}                    # 50 MB: written in full
+    assert a["link.npy"].dtype == np.float32 and a["match.npy"].dtype == np.float64
+    assert np.array_equal(a["match.npy"], per_pair["match"].numpy()) and np.array_equal(a["link.npy"], per_pair["link"].numpy())
+    big = {"link": torch.cat([per_pair["link"]] * 2)}
+    for d in ("c", "d"):
+        bench.dump_outputs(str(tmp_path / d), [("", big, shared, 2 * B)])
+    idx = np.load(tmp_path / "c" / "pair_index.npy")
+    assert 0 < len(idx) < 2 * B and np.array_equal(idx, np.load(tmp_path / "d" / "pair_index.npy"))
+    assert np.array_equal(np.load(tmp_path / "c" / "link.npy"), big["link"].numpy()[idx.astype(np.int64)])
+    assert sum(os.path.getsize(tmp_path / "c" / f) for f in os.listdir(tmp_path / "c")) <= bench.DUMP_LIMIT
+
+
+@pytest.mark.gpu
+def test_dump_outputs_of_the_timed_path_repeat_exactly(tmp_path):
+    """bench.py --dump-outputs on a small cfg4 batch, twice: the same seeded inputs give the same outputs bit for bit, and
+    the files are what predict_batch returns (per-pair scores, assignments and match indices, trans, status)."""
+    import numpy as np
+    outs = []
+    for run in ("a", "b"):
+        r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--steps", "2", "--warmup", "0", "--pairs", "2",
+                            "--no-cpu", "--dump-outputs", str(tmp_path / run)], capture_output=True, text=True, timeout=900)
+        assert r.returncode == 0, r.stderr[-2000:]
+        assert json.loads(r.stdout.strip().splitlines()[-1])["steps"] == 2
+        outs.append({f[:-4]: np.load(tmp_path / run / f) for f in os.listdir(tmp_path / run)})
+    a, b = outs
+    assert set(a) == {"det", "link", "new", "end", "assign_det", "assign_link", "assign_new", "assign_end", "match", "trans1",
+                      "trans2", "status"}
+    assert a["link"].shape == (2, 3, 128, 128) and a["link"].dtype == np.float32 and a["match"].shape == (2, 128)
+    assert a["status"][0] == 0 and np.all((a["match"] >= -1) & (a["match"] < 128))
+    for k in a:
+        assert np.array_equal(a[k], b[k]), k

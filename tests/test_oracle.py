@@ -1,14 +1,15 @@
 """CPU: the oracle restatement against the golden fixtures produced by the UNMODIFIED reference
 (oracle/make_goldens.py), plus known-answer tests the reference never had (SURVEY §4)."""
 import numpy as np
+import os
 import types
 
 import pytest
 import torch
 
-from helpers import case_tol, golden_cases, relerr
+from helpers import GOLDEN_DIR, case_tol, golden_cases, relerr
 from mmmot_b200.synthetic import synthetic_pair, synthetic_state_dict
-from oracle import lp_ref, ref_loader, torch_ref
+from oracle import lp_ref, torch_ref
 
 CASES = golden_cases()
 
@@ -46,15 +47,16 @@ def test_stn_is_input_independent_constant(g):
     assert relerr(stn_constant(sd, "point_net.feat.stn2", 64).float(), g["trans2"][0]) < 1e-6
 
 
-@pytest.mark.skipif(not ref_loader.available(), reason="/root/reference not present (GPU box)")
 def test_oracle_vs_live_reference_cfg1():
-    """BASELINE config[0]: Fusion-A, N=8 plumbing case, live against the imported reference."""
-    from oracle.make_goldens import reference_forward
-    case = ("live", "A", "multiply", "none", 0.2, 8, 8, 64, 64, False, 21)
-    ref = reference_forward(case)
-    sd = synthetic_state_dict("A", seed=21)
-    dets, info, split = synthetic_pair(8, 8, 64, 64, seed=21)
-    det, link, new, end, _ = torch_ref.forward(sd, dets, info, split, "A", "multiply", "none", 0.2)
+    """BASELINE config[0]: Fusion-A, N=8 plumbing case at 64x64 crops, against the outputs the unmodified reference
+    computed for it (oracle/make_goldens.py::live_golden)."""
+    from oracle.make_goldens import LIVE_CASE
+    name, fusion, op, sm, thr, n, m, pts, hw, ragged, seed = LIVE_CASE
+    g = np.load(os.path.join(GOLDEN_DIR, name + ".npz"))
+    ref = {k: torch.from_numpy(g[k]) for k in ("det", "link", "new", "end")}
+    sd = synthetic_state_dict(fusion, seed=seed)
+    dets, info, split = synthetic_pair(n, m, pts, hw, seed=seed, ragged=ragged)
+    det, link, new, end, _ = torch_ref.forward(sd, dets, info, split, fusion, op, sm, thr)
     assert relerr(link[0], ref["link"]) < 1e-4 and relerr(det, ref["det"]) < 1e-4
     assert relerr(new, ref["new"]) < 1e-4 and relerr(end, ref["end"]) < 1e-4
 
