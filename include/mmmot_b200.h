@@ -287,17 +287,11 @@ int mmmot_set_engine(int engine);
  * 72 only the K = 4608 layers (6.8e-5). */
 int mmmot_set_kseg(int chunks);
 
-/* Profiling / A-B experiments (tools/stage_times.py, TC_DBG=...).  Results are WRONG with any of bits 0-3 set;
- * the other bits select an alternative implementation of the same arithmetic.  Default 0.
+/* Profiling experiments on the tcgen05 kernels (tools/stage_times.py, TC_DBG=...): each bit removes one part of
+ * the work to show what bounds a kernel, so results are WRONG with any bit set.  Default 0.
  *   bit 0 (1)    skip epilogue work          bit 1 (2)   skip weight loads
  *   bit 2 (4)    skip operand loads          bit 3 (8)   skip MMA issue
- *   bit 4 (16)   two 128-row subtiles per tile also for short K chains (no TMEM double buffering)
- *   bit 5 (32)   first VGG layer as the direct FP32 FFMA kernel instead of im2col + tensor cores
- *   bit 6 (64)   64-channel layers on the channel-major kernel instead of the pixel-major one
- *   bit 7 (128)  pixel-major epilogue with 128-bit instead of 256-bit stores
- *   bit 8 (256)  pixel-major kernel without halo boxes (nine boxes per channel chunk)
- *   bit 9 (512)  no fused max-pool in the pixel-major epilogue
- *   bit 14 (16384) first VGG layer with a separate im2col pre-pass instead of in-kernel operand producers */
+ * Returns MMMOT_E_ARG, leaving the flags unchanged, if any other bit is set. */
 int mmmot_set_debug(int flags);
 
 /* Test hook: Y[M][S] = W X + bias through the FP32 FFMA engine (engine must be 1); Wt is [K][M] fp32, X is [K][S],

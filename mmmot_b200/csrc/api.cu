@@ -170,7 +170,11 @@ namespace { int g_engine = 0; int g_dbg = 0; int g_kseg = 36; }
 int mm_kseg_chunks() { return g_kseg; }
 extern "C" int mmmot_set_kseg(int chunks) { if (chunks < 0) return MMMOT_E_ARG; g_kseg = chunks; return 0; }
 int mm_debug_flags() { return g_dbg; }
-extern "C" int mmmot_set_debug(int flags) { g_dbg = flags; return 0; }
+extern "C" int mmmot_set_debug(int flags) {
+  if (flags & ~15) return MMMOT_E_ARG;
+  g_dbg = flags;
+  return 0;
+}
 
 int mm_engine() { return g_engine; }
 

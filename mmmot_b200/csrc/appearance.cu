@@ -101,81 +101,6 @@ __global__ void pool_sum_mean_kernel(const unsigned long long* __restrict__ sum,
   if (idx < n) out[idx] = (float)((double)sum[idx] * (1.0 / 4294967296.0) * (double)inv_hw);
 }
 
-// First VGG layer (3 -> 64, K = 27) of the tensor-core trunk: too thin for the MMA path (memory-bound: 1 MB of
-// output per crop), so a direct FP32 FFMA kernel writes the FP16 hi/lo NHWC planes the next layer's TMA loads
-// read.  Each thread: 2 horizontally adjacent pixels x 16 channels (weights from smem as 128-bit loads);
-// CTA = 64 pixel pairs x 4 channel groups.  wt: [(ky*3+kx)*3 + ci][64] (BN folded), ReLU fused.  W % 2 == 0.
-__global__ void __launch_bounds__(256, 4) conv0_packed_kernel(const float* __restrict__ in, const float* __restrict__ wt,
-                                                              const float* __restrict__ bias, long n_pairs, int H, int W,
-                                                              __half* __restrict__ out, long plane, int* status) {
-  __shared__ __align__(16) float ws[27 * 64];
-  __shared__ float bs[64];
-  for (int i = threadIdx.x; i < 27 * 64; i += 256) ws[i] = wt[i];
-  if (threadIdx.x < 64) bs[threadIdx.x] = bias[threadIdx.x];
-  __syncthreads();
-  // warp-uniform channel group (weight reads are smem broadcasts); lanes = 32 consecutive pixel pairs
-  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  const long pr = (long)blockIdx.x * 64 + (warp >> 2) * 32 + lane;
-  const int cg = (warp & 3) * 16;
-  if (pr >= n_pairs) return;
-  const int wp = W >> 1, hw = H * W;
-  const long row = pr / wp;                // (img, y)
-  const int x0 = (int)(pr - row * wp) * 2;
-  const long img = row / H;
-  const int y = (int)(row - img * H);
-  const float* src = in + img * 3 * hw;
-  float acc[2][16];
-#pragma unroll
-  for (int p = 0; p < 2; p++)
-#pragma unroll
-    for (int c = 0; c < 16; c++) acc[p][c] = bs[cg + c];
-#pragma unroll
-  for (int ci = 0; ci < 3; ci++) {
-#pragma unroll
-    for (int ky = 0; ky < 3; ky++) {
-      const int yy = y + ky - 1;
-      const bool oky = yy >= 0 && yy < H;
-      const float* rowp = src + (long)ci * hw + (long)yy * W + x0;
-      float v[4];
-#pragma unroll
-      for (int t = 0; t < 4; t++) {
-        const int xx = x0 + t - 1;
-        v[t] = (oky && xx >= 0 && xx < W) ? __ldg(rowp + t - 1) : 0.f;
-      }
-#pragma unroll
-      for (int kx = 0; kx < 3; kx++) {
-        const float4* wr = reinterpret_cast<const float4*>(ws + ((ky * 3 + kx) * 3 + ci) * 64 + cg);
-#pragma unroll
-        for (int q = 0; q < 4; q++) {
-          const float4 t4 = wr[q];
-#pragma unroll
-          for (int p = 0; p < 2; p++) {
-            acc[p][4 * q] = fmaf(v[p + kx], t4.x, acc[p][4 * q]);
-            acc[p][4 * q + 1] = fmaf(v[p + kx], t4.y, acc[p][4 * q + 1]);
-            acc[p][4 * q + 2] = fmaf(v[p + kx], t4.z, acc[p][4 * q + 2]);
-            acc[p][4 * q + 3] = fmaf(v[p + kx], t4.w, acc[p][4 * q + 3]);
-          }
-        }
-      }
-    }
-  }
-  const long pix0 = row * W + x0;
-#pragma unroll
-  for (int p = 0; p < 2; p++) {
-    __half h[16], l[16];
-#pragma unroll
-    for (int c = 0; c < 16; c++) {
-      tma::split_f16(fmaxf(acc[p][c], 0.f), h[c], l[c]);
-      mm_range_flag(status, acc[p][c]);
-    }
-    __half* dst = out + (pix0 + p) * 64 + cg;
-    reinterpret_cast<uint4*>(dst)[0] = reinterpret_cast<uint4*>(h)[0];
-    reinterpret_cast<uint4*>(dst)[1] = reinterpret_cast<uint4*>(h)[1];
-    reinterpret_cast<uint4*>(dst + plane)[0] = reinterpret_cast<uint4*>(l)[0];
-    reinterpret_cast<uint4*>(dst + plane)[1] = reinterpret_cast<uint4*>(l)[1];
-  }
-}
-
 // First VGG layer on the tensor cores: the 3-channel fp32 NCHW crop is expanded to the 27 (+5 zero) taps of every
 // pixel, k = ci*9 + ky*3 + kx, as FP16 hi/lo planes [2][pixels][32]; the layer is then a K=32 contraction on the TMA
 // engine whose epilogue writes the NHWC planes conv 1 reads.  One thread per pixel, 64 B per plane.
@@ -302,6 +227,8 @@ extern "C" int mmmot_appearance_fwd(const mmmot_weights* wts, const float* crops
   // take the same path and stay bit-identical
   const bool tc_trunk = mm_engine() == 2 || (mm_engine() == 0 && (long)L * H * W >= 32768);
   if (tc_trunk) {
+    // the 64-channel layers 0 and 1 run on the pixel-major kernel, which reads the compact weight tiles
+    if (!wts->w[MMMOT_W_VGG_WPX0] || !wts->w[MMMOT_W_VGG_WPX0 + 1]) return MMMOT_E_ARG;
     __half* hb[2] = {reinterpret_cast<__half*>(buf[0]), reinterpret_cast<__half*>(buf[1])};
     const __half* cur = nullptr;
     long cur_plane = 0;
@@ -318,16 +245,12 @@ extern "C" int mmmot_appearance_fwd(const mmmot_weights* wts, const float* crops
                                  4.0 * (double)n_img * h * w * (cin + (i == 1 ? cout / 4.0 : cout)));
       if (i == 0) {
         const long n_pix = (long)n_img * h * w;
-        if (mm_debug_flags() & 32) {   // A/B: direct FP32 FFMA first layer
-          conv0_packed_kernel<<<mm_cdiv(n_pix / 2, 64), 256, 0, st>>>(crops, wts->w[MMMOT_W_VGG_WT0], wts->w[MMMOT_W_VGG_B0],
-                                                                     n_pix / 2, h, w, hb[which], plane_out, status);
-          MM_LAUNCH_CHECK();
-        } else if (wts->w[MMMOT_W_VGG_WPX0] && !(mm_debug_flags() & 16384) && ((long)h * w) % 256 == 0 && w <= 512) {
+        if (gemm_tma_px_gen27_fits(h, w)) {
           // taps generated inside the contraction kernel (no im2col matrix in HBM)
           MM_TRY(gemm_tma_px_launch_gen27(crops, n_img, h, w, (const uint4*)wts->w[MMMOT_W_VGG_WPX0],
                                           wts->tc_scale[MMMOT_W_VGG_WP0], wts->w[MMMOT_W_VGG_B0], hb[which], plane_out,
                                           status, st));
-        } else {
+        } else {   // crops too wide for the in-kernel staging
           if (n_pix >= (1L << 31)) return MMMOT_E_SHAPE;
           __half* cols = hb[which ^ 1];   // [2][pixels][32] taps, dead once the contraction has run
           im2col27_kernel<<<mm_cdiv(n_pix, 256), 256, 0, st>>>(crops, n_pix, h, w, cols, n_pix * 32, status);

@@ -54,9 +54,9 @@ __device__ __forceinline__ void ld_global_256(const float* p, float (&v)[8]) {
 }
 
 // PAIRED: software-pipelined producers (the next chunk's source vectors are loaded before the current chunk is
-// converted).  GEN_PAIR_*: only for m == 128, where a 256-column tile is two whole rows i and the thread's four items are
-// {row i0, row i0 + 1} x {j = cb, j = cb + 64}: 2 + 2 source vectors instead of 4 + 4, which leaves the registers.
-// GEN_NORM: any shape; the GroupNorm affine is then re-read from shared memory per pair of items.
+// converted).  GEN_COPY: always.  GEN_PAIR_*: only for m == 128, where a 256-column tile is two whole rows i and the
+// thread's four items are {row i0, row i0 + 1} x {j = cb, j = cb + 64}: 2 + 2 source vectors instead of 4 + 4, which
+// leaves the registers.  GEN_NORM: never; it holds the chunk's GroupNorm affine in registers instead.
 template <int GEN, bool PAIRED>
 static __global__ void __launch_bounds__(G_THREADS, 1) gemm_gen_kernel(const GenP P) {
   const GemmP& p = P.t.g;
@@ -302,9 +302,7 @@ static __global__ void __launch_bounds__(G_THREADS, 1) gemm_gen_kernel(const Gen
             float x[8];
             if (GEN == GEN_NORM) {
               const float(&y)[8] = R.a[r];
-              // prefetching variant: the affine is re-read from shared memory per pair of items (volatile asm) instead
-              // of holding the eight (scale, shift) pairs across the chunk: 16 registers for the prefetched vectors
-              if (!PAIRED ? r == 0 : !(r & 1)) { lds128(sca, sc0); lds128(sca + 16, sc1); lds128(sha, sh0); lds128(sha + 16, sh1); }
+              if (r == 0) { lds128(sca, sc0); lds128(sca + 16, sc1); lds128(sha, sh0); lds128(sha + 16, sh1); }
               x[0] = fmaxf(fmaf(y[0], sc0.x, sh0.x), 0.f); x[1] = fmaxf(fmaf(y[1], sc0.y, sh0.y), 0.f);
               x[2] = fmaxf(fmaf(y[2], sc0.z, sh0.z), 0.f); x[3] = fmaxf(fmaf(y[3], sc0.w, sh0.w), 0.f);
               x[4] = fmaxf(fmaf(y[4], sc1.x, sh1.x), 0.f); x[5] = fmaxf(fmaf(y[5], sc1.y, sh1.y), 0.f);
@@ -404,8 +402,13 @@ static int gemm_gen_launch_t(const GemmP& g, const uint4* Wp, float out_scale, c
 template <int GEN>
 static int gemm_gen_launch(const GemmP& g, const uint4* Wp, float out_scale, const float* src, int ld_src,
                            const float* gsc, const float* gsh, int n, int m, int Lf, cudaStream_t st) {
-  // debug bit 10 (1024): producers without the software pipeline (A/B runs)
-  const bool pipe = !(mm_debug_flags() & 1024) && (GEN == gen::GEN_NORM ? (mm_debug_flags() & 4096) != 0 : GEN == gen::GEN_COPY ? true : m == 128);
-  if (pipe) return gemm_gen_launch_t<GEN, true>(g, Wp, out_scale, src, ld_src, gsc, gsh, n, m, Lf, st);
-  return gemm_gen_launch_t<GEN, false>(g, Wp, out_scale, src, ld_src, gsc, gsh, n, m, Lf, st);
+  // PAIRED as documented at gemm_gen_kernel
+  if constexpr (GEN == gen::GEN_NORM)
+    return gemm_gen_launch_t<GEN, false>(g, Wp, out_scale, src, ld_src, gsc, gsh, n, m, Lf, st);
+  else if constexpr (GEN == gen::GEN_COPY)
+    return gemm_gen_launch_t<GEN, true>(g, Wp, out_scale, src, ld_src, gsc, gsh, n, m, Lf, st);
+  else if (m == 128)
+    return gemm_gen_launch_t<GEN, true>(g, Wp, out_scale, src, ld_src, gsc, gsh, n, m, Lf, st);
+  else
+    return gemm_gen_launch_t<GEN, false>(g, Wp, out_scale, src, ld_src, gsc, gsh, n, m, Lf, st);
 }

@@ -41,14 +41,12 @@ struct TmaP {
   long plane_elems;         // output: distance (in fp16 elements) between the hi and lo planes
   int ksegs, kc_per_seg;    // conv: K is accumulated in `ksegs` TMEM passes of kc_per_seg chunks whose fp32
   float* acc_scratch;       // partial sums are combined in fp32 RN through acc_scratch[pixel][M] (see launcher)
-  int halo, pool;           // halo: pixel-major kernel only (gemm_tma_px.cuh), vertical taps from one halo box
-                            // pool: fused 2x2 max-pool in the conv epilogue (both kernels): the pooled map is written
+  int pool;                 // fused 2x2 max-pool in the conv epilogue (both kernels): the pooled map is written
   unsigned long long* pool_sum;   // channel-major conv + pool: if set, the pooled values are also summed per (image, channel)
                             // into pool_sum[img][M] as 2^-32 fixed point (SkipPool's global average, order-independent)
   unsigned long long* segsum;   // matrix mode: if set, nothing is stored; relu(x*sc[g][co] + sh[g][co]) is summed per
                             // detection (g.seg[column]) into segsum[det][M] as 2^-32 fixed point (order-independent)
   int* status;              // workspace status word (FP16 range flag of the planar outputs) or null
-  int wcompact;             // pixel-major kernel: t.Wp holds the compact N = 64 tiles (8 KB per k chunk, weights.py::pack_px)
   const float* gen_src;     // pixel-major kernel, GEN27 variant: fp32 NCHW 3-channel crops [n_img][3][H][W]; the 27 (+5 zero)
                             // taps of every pixel (k = ci*9 + ky*3 + kx) are built in shared memory by producer warps
   const int4* chunk_tab;    // matrix mode with g.seg: per (column tile, half) the four 32-column chunks' descriptors
@@ -624,7 +622,8 @@ static inline int make_map_4d(CUtensorMap* m, const void* basep, int n_img, int 
 
 #include "gemm_tma_px.cuh"
 
-// pixel-major kernel for 64-channel planar outputs (see gemm_tma_px.cuh); P fully prepared by the caller
+// pixel-major kernel for 64-channel planar outputs (see gemm_tma_px.cuh); P fully prepared by the caller, P.t.Wp = the
+// compact N = 64 weight tiles (weights.py::pack_px)
 static int gemm_tma_px_launch(tma::TmaP& P, const CUtensorMap& mh, const CUtensorMap& ml, int sms, cudaStream_t st) {
   static std::atomic<unsigned long long> attr{0};
   MM_TRY(mm_ensure_smem(tma::gemm_tma_px_kernel<false>, tma::PX_SMEM_BYTES, attr));
@@ -638,12 +637,17 @@ static int gemm_tma_px_launch(tma::TmaP& P, const CUtensorMap& mh, const CUtenso
 // First VGG layer (3 -> 64 channels, 3x3 / pad 1) straight from the fp32 NCHW crops: the K = 32 operand (27 taps + 5
 // zeros per pixel, FP16 hi/lo) is generated in shared memory by the kernel's producer warps, so the im2col matrix
 // (128 B per pixel written and read back) never exists.  Output: planar FP16 NHWC, bias + ReLU applied.
+// Crop shapes it takes: a tile = 256 consecutive pixels of one image, and the tile's neighbourhood, (256 + 2W + 2) x 3
+// floats, is staged in two 8 KB weight slots.  Wider crops need the im2col27 pre-pass.
+constexpr int PX_GEN27_MAX_W = 512;
+static_assert((tc::BN + 2 * PX_GEN27_MAX_W + 2) * 12 <= 2 * tma::PX_W_SLOT, "GEN27 staging buffer");
+static inline bool gemm_tma_px_gen27_fits(int H, int W) { return ((long)H * W) % tc::BN == 0 && W <= PX_GEN27_MAX_W; }
+
 static int gemm_tma_px_launch_gen27(const float* crops, int n_img, int H, int W, const uint4* Wpx, float out_scale,
                                     const float* bias, __half* Yhi, long y_plane, int* status, cudaStream_t st) {
   if (!crops || !Wpx || !Yhi) return MMMOT_E_ARG;
   const long n_pix = (long)n_img * H * W;
-  // a tile = 256 consecutive pixels of one image; staging buffer (256 + 2W + 2) x 3 floats in two 8 KB weight slots
-  if (n_pix >= (1L << 31) || ((long)H * W) % tc::BN || (tc::BN + 2 * W + 2) * 12 > 2 * tma::PX_W_SLOT) return MMMOT_E_SHAPE;
+  if (n_pix >= (1L << 31) || !gemm_tma_px_gen27_fits(H, W)) return MMMOT_E_SHAPE;
   int sms = 0;
   MM_TRY(mm_sm_count(&sms));
   static std::atomic<unsigned long long> attr{0};
@@ -655,7 +659,7 @@ static int gemm_tma_px_launch_gen27(const float* crops, int n_img, int H, int W,
   g.S = (int)n_pix; g.tiles_per_group = mm_cdiv(n_pix, tc::BN); g.num_tiles = g.tiles_per_group;
   g.Y = reinterpret_cast<float*>(Yhi); g.y_ms = 64;
   P.t.g = g;
-  P.t.Wp = Wpx; P.wcompact = 1;
+  P.t.Wp = Wpx;
   P.t.m_tiles = 1; P.t.k_chunks = 1; P.t.mt_per_cta = 1;
   P.t.out_scale = out_scale;
   P.t.out_mode = tma::OUT_PLANAR;
@@ -675,6 +679,8 @@ static int gemm_tma_px_launch_gen27(const float* crops, int n_img, int H, int W,
 
 // 1x1 contraction on planar FP16 (hi, lo) channels-last activations X_hi[rows][ldx], X_lo = X_hi + x_plane.
 // g: M, K (multiple of 32), bias, tiles, x_gs (rows per group), Y / y_ms / y_gs, part, addend...
+// Wpx: the same weights as compact N = 64 tiles (weights.py::pack_px); given those, a plain 64-channel planar output
+// runs on the pixel-major kernel.
 static int gemm_tma_launch_mat(const GemmP& g, const uint4* Wp, float out_scale, const __half* Xhi, long x_plane,
                                long rows, int ldx, int out_mode, long y_plane, cudaStream_t st,
                                unsigned long long* segsum = nullptr, int* status = nullptr, const int4* chunk_tab = nullptr,
@@ -693,7 +699,7 @@ static int gemm_tma_launch_mat(const GemmP& g, const uint4* Wp, float out_scale,
   // two 128-row subtiles per CTA share each operand box; short K chains (<= 16 chunks) are epilogue-bound instead,
   // so they run one subtile per tile and double-buffer the accumulator in TMEM (epilogue overlaps the next MMAs).
   // The arithmetic of a subtile does not depend on this choice.
-  P.t.mt_per_cta = (P.t.m_tiles >= 2 && (P.t.k_chunks > 16 || (mm_debug_flags() & 16))) ? 2 : 1;
+  P.t.mt_per_cta = (P.t.m_tiles >= 2 && P.t.k_chunks > 16) ? 2 : 1;
   P.t.out_scale = out_scale;
   P.t.out_mode = out_mode;
   P.t.dbg = mm_debug_flags();
@@ -706,9 +712,8 @@ static int gemm_tma_launch_mat(const GemmP& g, const uint4* Wp, float out_scale,
   alignas(64) CUtensorMap mh, ml;
   MM_TRY(tma::make_map_2d(&mh, Xhi, rows, g.K, ldx));
   MM_TRY(tma::make_map_2d(&ml, Xhi + x_plane, rows, g.K, ldx));
-  if (out_mode == tma::OUT_PLANAR && g.M == 64 && g.y_ms == 64 && !g.part && !segsum && !g.addend && !g.tile_tab &&
-      !(P.t.dbg & 64)) {
-    if (Wpx) { P.t.Wp = Wpx; P.wcompact = 1; }
+  if (Wpx && out_mode == tma::OUT_PLANAR && g.M == 64 && g.y_ms == 64 && !g.part && !segsum && !g.addend && !g.tile_tab) {
+    P.t.Wp = Wpx;
     return gemm_tma_px_launch(P, mh, ml, sms, st);
   }
   const long mgroups = (P.t.m_tiles + P.t.mt_per_cta - 1) / P.t.mt_per_cta;
@@ -744,31 +749,29 @@ static int gemm_tma_launch_conv(const GemmP& g0, const uint4* Wp, float out_scal
         if (waste < best - 1e-9) { best = waste; bx = cx; by = cy; bi = ci; }
       }
   }
-  // 64-channel outputs run on the pixel-major kernel (gemm_tma_px.cuh); it prefers a 16 x 16 single-image box
-  // (vertical taps from one halo box, 2x2 pooling windows inside a warp) when that wastes no more than the best box
+  // 64-channel outputs with compact weights run on the pixel-major kernel (gemm_tma_px.cuh) when a 16 x 16
+  // single-image box (vertical taps from one halo box, 2x2 pooling windows inside a warp) wastes no more than the best
+  // box; for H and W multiples of 16 it always does
   const int seg_chunks = mm_kseg_chunks();   // 0 = single pass
-  const int dbg = mm_debug_flags();
-  const bool px = g0.M == 64 && !g0.part && !(dbg & 64) && !(acc_scratch && seg_chunks > 0 && 9 * C / tc::BK > seg_chunks);
+  bool px = Wpx && g0.M == 64 && !g0.part && !(acc_scratch && seg_chunks > 0 && 9 * C / tc::BK > seg_chunks);
   if (px) {
     const double best = (double)mm_cdiv(W, bx) * bx / W * mm_cdiv(H, by) * by / H * mm_cdiv(n_img, bi) * bi / n_img;
     const double w16 = (double)mm_cdiv(W, 16) * 16 / W * mm_cdiv(H, 16) * 16 / H;
-    if (w16 <= best + 1e-9) { bx = 16; by = 16; bi = 1; }
+    px = w16 <= best + 1e-9;
+    if (px) { bx = 16; by = 16; bi = 1; }
   }
   tma::TmaP P;
   memset(&P, 0, sizeof(P));
   GemmP g = g0;
   g.K = 9 * C;
   P.conv = 1; P.bx = bx; P.by = by; P.bi = bi;
-  if (px) {
-    P.halo = (bi == 1 && bx >= 8 && bx * (by + 2) * 64 <= tma::PX_X_PLANE && !(dbg & 256)) ? 1 : 0;
-    if (y_plane_pooled > 0 && did_pool && bx >= 2 && bx <= 16 && by >= 2 && !(H & 1) && !(W & 1) && !(dbg & 512)) {
-      P.pool = 1;
-      *did_pool = 1;
-    }
+  if (px && y_plane_pooled > 0 && did_pool && !(H & 1) && !(W & 1)) {
+    P.pool = 1;
+    *did_pool = 1;
   }
   // channel-major kernel: the 2x2 max-pool (and SkipPool's per-image sums) fused into the epilogue when every pooling
   // window lies inside one thread's chunks: box rows of <= 32 pixels, an even number of box rows per 128-column half
-  if (!px && y_plane_pooled > 0 && did_pool && bx >= 2 && bx <= 32 && by >= 2 && !(H & 1) && !(W & 1) && !(dbg & 512)) {
+  if (!px && y_plane_pooled > 0 && did_pool && bx >= 2 && bx <= 32 && by >= 2 && !(H & 1) && !(W & 1)) {
     P.pool = 1;
     P.pool_sum = pool_sum;
     *did_pool = 1;
@@ -796,11 +799,11 @@ static int gemm_tma_launch_conv(const GemmP& g0, const uint4* Wp, float out_scal
     P.acc_scratch = acc_scratch;
   }
   alignas(64) CUtensorMap mh, ml;
-  const int box_y = P.halo ? by + 2 : by;
+  const int box_y = px ? by + 2 : by;   // pixel-major: halo box of the three vertical taps
   MM_TRY(tma::make_map_4d(&mh, Xhi, n_img, H, W, C, bx, box_y, bi));
   MM_TRY(tma::make_map_4d(&ml, Xhi + x_plane, n_img, H, W, C, bx, box_y, bi));
   if (px) {
-    if (Wpx) { P.t.Wp = Wpx; P.wcompact = 1; }
+    P.t.Wp = Wpx;
     return gemm_tma_px_launch(P, mh, ml, sms, st);
   }
   const long mgroups = (P.t.m_tiles + P.t.mt_per_cta - 1) / P.t.mt_per_cta;

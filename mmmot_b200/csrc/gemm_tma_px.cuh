@@ -3,22 +3,22 @@
 // With Cout = 64 the channel-major kernel (gemm_tma.cuh) pads the MMA's M from 64 to 128 — half of every
 // tensor-core instruction is zeros and half of the epilogue warps cannot reach any valid TMEM lane.  Here the
 // roles are swapped: the 256-pixel activation box is the A operand (two M=128 subtiles, K-major SWIZZLE_64B, as
-// TMA writes it) and the packed weights are the B operand (N = 64, K-major canonical layout, only rows 0..63 of
-// the packed tile are fetched).  D[pixel][channel] lives in TMEM lanes = pixels, so all eight epilogue warps work,
-// every thread owns 32 consecutive channels of one pixel and stores its 64 bytes per plane directly — no shared-
-// memory transpose.  Two 128-column accumulator buffers: the epilogue of tile i overlaps the MMAs of tile i+1.
+// TMA writes it) and the compact weight tiles (below) are the B operand.  D[pixel][channel] lives in TMEM lanes =
+// pixels, so all eight epilogue warps work, every thread owns 32 consecutive channels of one pixel and stores its 64
+// bytes per plane directly — no shared-memory transpose.  Two 256-column accumulator buffers: the epilogue of tile i
+// overlaps the MMAs of tile i+1.
 // Same arithmetic as the channel-major kernel: FP16 hi/lo split operands, D += Xhi*Whi + Xhi*Wlo + Xlo*Whi.
 #pragma once
 
 namespace tma {
 
-// Halo mode (3x3 conv, one image per box): a stage holds the (by+2)-row box of ONE horizontal tap and channel chunk;
-// its three vertical taps are the same shared-memory box read at start addresses dy*bx*64 B (whole swizzle atoms for
-// bx >= 8), so the activation traffic from L2 — what bounds this layer — drops from 9 to 3*(by+2)/by boxes per
-// chunk.  Optional fused 2x2 max-pool: with bx <= 16 a warp's 32 pixels are whole pooling windows (lanes l, l^1,
-// l^bx, l^(bx+1)), so the pooled NHWC planes are written directly and the full-resolution activation never exists.
-constexpr int PX_W_SLOT = 8192;                 // compact weight tile: [hi|lo][k group 4][row group 8][8][8] f16
-constexpr int PX_W_LBO = 1024;
+// Conv mode (3x3 conv, 16 x 16 single-image box): a stage holds the (by+2)-row halo box of ONE horizontal tap and
+// channel chunk; its three vertical taps are the same shared-memory box read at start addresses dy*bx*64 B (whole
+// swizzle atoms for bx >= 8), so the activation traffic from L2 — what bounds this layer — drops from 9 to
+// 3*(by+2)/by boxes per chunk.  Optional fused 2x2 max-pool: with bx <= 16 a warp's 32 pixels are whole pooling windows
+// (lanes l, l^1, l^bx, l^(bx+1)), so the pooled NHWC planes are written directly and the full-resolution activation
+// never exists.
+constexpr int PX_W_SLOT = 8192;                 // one k chunk of the compact weight tiles (below)
 constexpr int PX_X_OFF = 3 * PX_W_SLOT;         // 24 KB: three tap slots
 constexpr int PX_X_PLANE = 24576;               // up to 384 box rows x 64 B per plane
 constexpr int PX_STAGE = PX_X_OFF + 2 * PX_X_PLANE;   // 72 KB
@@ -58,11 +58,10 @@ gemm_tma_px_kernel(const TmaP P, const __grid_constant__ CUtensorMap map_hi, con
 
   const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
   const long total_tiles = p.num_tiles;
-  const int KC = P.t.k_chunks;
-  const int cchunks = P.conv ? P.C / BK : KC;
-  const int ntap = P.halo ? 3 : 1;                       // vertical taps served by one stage
-  const int nstage = P.halo ? 3 * cchunks : KC;          // stages per tile
-  const uint32_t xbytes = P.halo ? (uint32_t)(P.bx * (P.by + 2) * 64) : (uint32_t)B_HALF;
+  const int cchunks = P.C / BK;                          // conv: channel chunks per tap
+  const int ntap = P.conv ? 3 : 1;                       // vertical taps served by one stage
+  const int nstage = P.conv ? 3 * cchunks : P.t.k_chunks;   // stages per tile
+  const uint32_t xbytes = P.conv ? (uint32_t)(P.bx * (P.by + 2) * 64) : (uint32_t)B_HALF;
 
   if (tid < 64) s_bias[tid] = p.bias ? p.bias[tid] : 0.f;
   if (tid == 0) {
@@ -100,8 +99,8 @@ gemm_tma_px_kernel(const TmaP P, const __grid_constant__ CUtensorMap map_hi, con
     const int lbx = 31 - __clz(max(P.bx, 1)), lby = 31 - __clz(max(P.by, 1));
     __half* yh = reinterpret_cast<__half*>(p.Y);
     uint32_t wcount = 0, racc = 0;   // racc: running max of the converted |hi| values (FP16 range guard)
-    for (long t = blockIdx.x; t < total_tiles; t += gridDim.x, wcount++) {
-      const int nt = (int)t;
+    // an int tile index (tile counts are < 2^31) keeps the GEN27 variant, at its 96-register cap, from spilling wcount
+    for (int nt = blockIdx.x; nt < total_tiles; nt += gridDim.x, wcount++) {
       int i0 = 0, y0 = 0, x0 = 0;
       if (P.conv) conv_origin(nt, i0, y0, x0);
       const int abuf = (int)(wcount & 1);
@@ -123,17 +122,12 @@ gemm_tma_px_kernel(const TmaP P, const __grid_constant__ CUtensorMap map_hi, con
           ok = row < p.S;
           o = row * 64 + cb;
         }
-        uint32_t v[32];
-        if (P.wcompact) {
-          // accumulator = columns [0, 64) (hi*hi + lo*hi) + columns [64, 128) (hi*lo partial)
-          uint32_t v2[32];
-          tmem_ld32(tmem_base + ((uint32_t)(q * 32) << 16) + (uint32_t)(abuf * 256 + sub * 128 + cb), v);
-          tmem_ld32(tmem_base + ((uint32_t)(q * 32) << 16) + (uint32_t)(abuf * 256 + sub * 128 + 64 + cb), v2);
+        // accumulator = columns [0, 64) (hi*hi + lo*hi) + columns [64, 128) (hi*lo partial)
+        uint32_t v[32], v2[32];
+        tmem_ld32(tmem_base + ((uint32_t)(q * 32) << 16) + (uint32_t)(abuf * 256 + sub * 128 + cb), v);
+        tmem_ld32(tmem_base + ((uint32_t)(q * 32) << 16) + (uint32_t)(abuf * 256 + sub * 128 + 64 + cb), v2);
 #pragma unroll
-          for (int j = 0; j < 32; j++) v[j] = __float_as_uint(__uint_as_float(v[j]) + __uint_as_float(v2[j]));
-        } else {
-          tmem_ld32(tmem_base + ((uint32_t)(q * 32) << 16) + (uint32_t)(abuf * 128 + sub * 64 + cb), v);
-        }
+        for (int j = 0; j < 32; j++) v[j] = __float_as_uint(__uint_as_float(v[j]) + __uint_as_float(v2[j]));
         if (P.t.dbg & 1) continue;
         if (P.pool) {
           // 2x2 max over lanes l, l^1 (x) and l^bx (y); bias + ReLU commute with the max and are applied below
@@ -193,20 +187,12 @@ gemm_tma_px_kernel(const TmaP P, const __grid_constant__ CUtensorMap map_hi, con
             if (row0 + px < p.S) st_global_256(dstp + (long)px * 64 + c * 8, w);
           }
           asm volatile("bar.sync %0, 64;" ::"r"(3 + q) : "memory");   // scratch free for the next subtile
-        } else if (ok && !(P.t.dbg & 128)) {
+        } else if (ok) {
           // 256-bit stores: every instruction writes whole 32-byte sectors (two per plane per thread)
           st_global_256(yh + o, hi);
           st_global_256(yh + o + 16, hi + 8);
           st_global_256(yh + o + P.plane_elems, lo);
           st_global_256(yh + o + P.plane_elems + 16, lo + 8);
-        } else if (ok) {
-          uint4* dh = reinterpret_cast<uint4*>(yh + o);
-          uint4* dl = reinterpret_cast<uint4*>(yh + o + P.plane_elems);
-#pragma unroll
-          for (int k = 0; k < 4; k++) {
-            dh[k] = make_uint4(hi[4 * k], hi[4 * k + 1], hi[4 * k + 2], hi[4 * k + 3]);
-            dl[k] = make_uint4(lo[4 * k], lo[4 * k + 1], lo[4 * k + 2], lo[4 * k + 3]);
-          }
         }
       }
       tc_fence_before();
@@ -236,19 +222,10 @@ gemm_tma_px_kernel(const TmaP P, const __grid_constant__ CUtensorMap map_hi, con
                 for (int ks = 0; ks < 2; ks++) {
                   const uint64_t x_hi = smem_desc_sw64(xo + sub * (128 * 64) + ks * 32);
                   const uint64_t x_lo = smem_desc_sw64(xo + PX_X_PLANE + sub * (128 * 64) + ks * 32);
-                  if (P.wcompact) {
-                    const uint64_t w_hl = smem_desc(wo + ks * 2 * PX_WC_LBO, PX_WC_LBO, SBO);   // rows 0-63 W_hi, 64-127 W_lo
-                    const uint32_t d = tmem_base + (uint32_t)(abuf * 256 + sub * 128);
-                    umma_f16(d, x_hi, w_hl, IDESC_N128, (si | ky | ks) ? 1u : 0u);
-                    umma_f16(d, x_lo, w_hl, IDESC_N64, 1u);
-                    continue;
-                  }
-                  const uint64_t w_hi = smem_desc(wo + ks * 2 * PX_W_LBO, PX_W_LBO, SBO);
-                  const uint64_t w_lo = smem_desc(wo + PX_W_SLOT / 2 + ks * 2 * PX_W_LBO, PX_W_LBO, SBO);
-                  const uint32_t d = tmem_base + (uint32_t)(abuf * 128 + sub * 64);
-                  umma_f16(d, x_hi, w_hi, IDESC_N64, (si | ky | ks) ? 1u : 0u);
-                  umma_f16(d, x_hi, w_lo, IDESC_N64, 1u);
-                  umma_f16(d, x_lo, w_hi, IDESC_N64, 1u);
+                  const uint64_t w_hl = smem_desc(wo + ks * 2 * PX_WC_LBO, PX_WC_LBO, SBO);   // rows 0-63 W_hi, 64-127 W_lo
+                  const uint32_t d = tmem_base + (uint32_t)(abuf * 256 + sub * 128);
+                  umma_f16(d, x_hi, w_hl, IDESC_N128, (si | ky | ks) ? 1u : 0u);
+                  umma_f16(d, x_lo, w_hl, IDESC_N64, 1u);
                 }
               }
             }
@@ -281,7 +258,7 @@ gemm_tma_px_kernel(const TmaP P, const __grid_constant__ CUtensorMap map_hi, con
       mbar_wait(empty_bar(s), ((it / STAGES) & 1) ^ 1);
       float* stg = reinterpret_cast<float*>(sm + s * PX_STAGE + PX_W_SLOT);
       const int lin0 = r0 - W - 1;
-      if (P.t.dbg & 4) {                         // A/B: no operand generation (results wrong)
+      if (P.t.dbg & 4) {                         // profiling: no operand generation (results wrong)
         __syncwarp();
         if (lane == 0) mbar_arrive(full_bar(s));
         continue;
@@ -353,28 +330,15 @@ gemm_tma_px_kernel(const TmaP P, const __grid_constant__ CUtensorMap map_hi, con
           mbar_wait(empty_bar(s), ((it / STAGES) & 1) ^ 1);
           mbar_expect_tx(full_bar(s), (uint32_t)ntap * PX_W_SLOT + (GEN27 ? 0u : 2u * xbytes));
           const uint32_t sw = base + s * PX_STAGE, sx = sw + PX_X_OFF;
-          const int kx = P.halo ? si / cchunks : 0, cc = P.halo ? si - kx * cchunks : 0;
+          const int kx = P.conv ? si / cchunks : 0, cc = P.conv ? si - kx * cchunks : 0;
           for (int ky = 0; ky < ntap; ky++) {
-            const int kc = P.halo ? (ky * 3 + kx) * cchunks + cc : si;
-            if (P.wcompact) {
-              // weights pre-packed for N = 64 (weights.py::pack_px): one 8 KB copy per k chunk
-              bulk_g2s(sw + ky * PX_W_SLOT, reinterpret_cast<const uint8_t*>(P.t.Wp) + (size_t)kc * PX_W_SLOT, PX_W_SLOT, full_bar(s));
-            } else {
-              // rows 0..63 of the packed [hi|lo][k group 4][row group 16][8][8] tile -> compact 8 KB slot: 8 runs of 1 KB
-              const uint8_t* src = reinterpret_cast<const uint8_t*>(P.t.Wp) + (size_t)kc * P.t.m_tiles * A_SUB;
-#pragma unroll
-              for (int r = 0; r < 8; r++)
-                bulk_g2s(sw + ky * PX_W_SLOT + r * PX_W_LBO, src + r * A_LBO, 1024, full_bar(s));
-            }
+            // weights pre-packed for N = 64 (weights.py::pack_px): one 8 KB copy per k chunk
+            const int kc = P.conv ? (ky * 3 + kx) * cchunks + cc : si;
+            bulk_g2s(sw + ky * PX_W_SLOT, reinterpret_cast<const uint8_t*>(P.t.Wp) + (size_t)kc * PX_W_SLOT, PX_W_SLOT, full_bar(s));
           }
-          if (P.halo) {
+          if (P.conv) {
             tma_load_4d(sx, &map_hi, cc * BK, x0 + kx - 1, y0 - 1, i0, full_bar(s));
             tma_load_4d(sx + PX_X_PLANE, &map_lo, cc * BK, x0 + kx - 1, y0 - 1, i0, full_bar(s));
-          } else if (P.conv) {
-            const int tap = si / cchunks, c2 = si - tap * cchunks;
-            const int dx = tap % 3 - 1, dy = tap / 3 - 1;
-            tma_load_4d(sx, &map_hi, c2 * BK, x0 + dx, y0 + dy, i0, full_bar(s));
-            tma_load_4d(sx + PX_X_PLANE, &map_lo, c2 * BK, x0 + dx, y0 + dy, i0, full_bar(s));
           } else if (!GEN27) {
             tma_load_2d(sx, &map_hi, si * BK, nt * BN, full_bar(s));
             tma_load_2d(sx + PX_X_PLANE, &map_lo, si * BK, nt * BN, full_bar(s));

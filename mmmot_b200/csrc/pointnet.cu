@@ -297,10 +297,9 @@ static int pointnet_impl(const mmmot_weights* wts, const float* points, const in
   const bool timed = mm_timing_on();
   if (use_tc) {
     // ---------------- tensor-core path: channels-last activations ----------------
-    // layer i writes fp32 Y[p][cout] + GroupNorm partials; norm_split turns it into the packed FP16
-    // operand of layer i+1.  y1's packed form (x1p) is kept for the head.
+    // layer i writes fp32 Y[p][cout] + GroupNorm partials.  Layers 3 and 4 read the previous layer's Y directly;
+    // layer 1's and layer 4's outputs become FP16 hi/lo planes (x1p, kept for the head; xp) for the TMA-fed kernel.
     float* ybuf[5] = {w.y1, w.t0, w.t1, w.t0, nullptr};
-    const bool gen_mid = !(mm_debug_flags() & 8192);   // debug bit 13: layers 3, 4 through norm_split + the TMA-fed kernel
     for (int i = 0; i < 5; i++) {
       const float* const* q = &wts->w[MMMOT_W_PN_L1 + 4 * i];
       GemmP p = gemm_defaults();
@@ -320,7 +319,7 @@ static int pointnet_impl(const mmmot_weights* wts, const float* points, const in
         // compulsory traffic: activation in (4 B per element) + fp32 activation out (none for the statistics pass)
         if (timed) mm_timing_begin(st, i == 4 ? MM_T_PN_L5A : MM_T_PN_L2 + (i - 1), 2.0 * cout[i] * cin[i] * cols,
                                    4.0 * (cin[i] + (i == 4 ? 0 : cout[i])) * cols);
-        if (gen_mid && (i == 2 || i == 3)) {
+        if (i == 2 || i == 3) {
           // layers 3, 4: GroupNorm + ReLU of the previous layer applied by this contraction's operand producers
           // (gemm_gen.cuh) straight from its fp32 output: no normalised copy is written
           MM_TRY((gemm_gen_launch<gen::GEN_NORM>(p, wp, wps, ybuf[i - 1], cin[i], w.sc, w.sh, 0, 0, 0, st)));
@@ -336,9 +335,9 @@ static int pointnet_impl(const mmmot_weights* wts, const float* points, const in
         pn_l1_apply_kernel<<<mm_cdiv(P * 16, 256), 256, 0, st>>>(points, q[0], q[1], w.sc, w.sh, w.seg, L, P, w.x1p, ar.status());
         MM_LAUNCH_CHECK();
         if (timed) mm_timing_end(st);
-      } else if (gen_mid && (i == 1 || i == 2)) {
+      } else if (i == 1 || i == 2) {
         // consumed in place by the next layer's producers
-      } else if (i < 4) {
+      } else if (i == 3) {
         if (timed) mm_timing_begin(st, MM_T_PN_NORM, 0.0, 8.0 * cout[i] * cols);
         MM_TRY(norm_split(ybuf[i], cout[i], w.sc, w.sh, cout[i], P, 0, w.seg, L, w.xp, st, ar.status()));
         if (timed) mm_timing_end(st);

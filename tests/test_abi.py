@@ -52,7 +52,20 @@ def test_workspace_queries_need_no_gpu(lib_built):
     assert lib.mmmot_lp_assign(None, 0, None, 0, None, 0, None, 0, 1, 1, 1, None, None, None, None, None, None, 0, None) == -1
 
 
-@pytest.mark.parametrize("fusion,nkeys,numel", [("C", 263, 21218212), ("A", 255, None), ("B", 259, None)])
+def test_set_debug_accepts_only_the_profiling_bits(lib_built):
+    """mmmot_set_debug takes bits 0-3 (skip epilogue / weight loads / operand loads / MMA issue) and refuses any other
+    bit, so a stale flag from a removed experiment fails instead of silently measuring the default path."""
+    lib = _lib.load()
+    try:
+        for flags in range(16):
+            assert lib.mmmot_set_debug(flags) == 0, flags
+        for flags in (16, 4096, 16384):
+            assert lib.mmmot_set_debug(flags) == -1, flags
+    finally:
+        lib.mmmot_set_debug(0)
+
+
+@pytest.mark.parametrize("fusion,nkeys,numel",[("C", 263, 21218212), ("A", 255, None), ("B", 259, None)])
 def test_state_dict_schema(fusion, nkeys, numel):
     """SURVEY §8b: 263 keys / 21 218 212 elements for Fusion C; key names are the drop-in contract."""
     sch = state_schema(fusion)

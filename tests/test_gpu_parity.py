@@ -170,10 +170,11 @@ def test_affinity_stage_matches_oracle(n, m, op, sm, engine):
         assert relerr(new[b], rn) < TOL and relerr(end[b], re) < TOL
 
 
-@pytest.mark.parametrize("hw,n", [(96, 3), (224, 1)])
+@pytest.mark.parametrize("hw,n", [(96, 3), (224, 1), (576, 1)])
 def test_non_power_of_two_crops(hw, n, engine):
     """Crop sizes that are multiples of 32 but not powers of two (224 is the reference's real crop size,
-    dataset/test_seq_dataset.py:217-218): partial TMA boxes / tile tails."""
+    dataset/test_seq_dataset.py:217-218): partial TMA boxes / tile tails.  576 is wider than the first VGG layer's
+    in-kernel operand producers stage (512), so the tcgen05 engine takes the im2col27 pre-pass there."""
     net, sd = make_net("A", "multiply", "none", 0.2, 12)
     dets, info, split = synthetic_pair(n, n, 32, hw, seed=50 + hw)
     o = net.forward_batch(dets.cuda(), info["points"][0].cuda(), info["points_split"][0], n, n, keep_feats=True)

@@ -1,5 +1,5 @@
 """Affinity stage alone (BASELINE cfg5): per-kernel device times from the library's tagged timing hook.
-Run on a GPU box:  python tools/aff_times.py [n] [pairs]      TC_DBG=0,4,8 runs the A/B bits of mmmot_set_debug."""
+Run on a GPU box:  python tools/aff_times.py [n] [pairs]      TC_DBG=0,4,8 runs with those mmmot_set_debug bits (0-3)."""
 import ctypes
 import os
 import sys
@@ -32,7 +32,7 @@ def main():
     g = torch.Generator(device="cuda").manual_seed(1)
     feats = torch.relu(torch.randn(pairs, 3, 512, 2 * n, device="cuda", generator=g))
     for dbg in [int(x) for x in os.environ.get("TC_DBG", "0").split(",")]:
-        lib.mmmot_set_debug(dbg)
+        _lib.check(lib.mmmot_set_debug(dbg), "mmmot_set_debug")
         for _ in range(2):
             net.associate_batch(feats, n)
         torch.cuda.synchronize()

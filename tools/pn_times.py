@@ -38,7 +38,7 @@ def main():
         _lib.check(lib.mmmot_pointnet_fwd(wts.ptr, vp(points), vp(split_d), ctypes.c_void_p(hs.ctypes.data), pairs, L, vp(feats),
                                           vp(ws), ws.numel(), st), "mmmot_pointnet_fwd")
     for dbg in [int(x) for x in os.environ.get("TC_DBG", "0").split(",")]:
-        lib.mmmot_set_debug(dbg)
+        _lib.check(lib.mmmot_set_debug(dbg), "mmmot_set_debug")
         for _ in range(2):
             run()
         torch.cuda.synchronize()

@@ -30,7 +30,7 @@ def main():
     split = torch.arange(0, B * L * pts + 1, pts, dtype=torch.int32)
     batch = (crops, points, split, n)
     lib = _lib.load()
-    lib.mmmot_set_debug(int(os.environ.get('TC_DBG', '0')))
+    _lib.check(lib.mmmot_set_debug(int(os.environ.get('TC_DBG', '0'))), "mmmot_set_debug")
     spans = collections.defaultdict(list)
     names = ["mmmot_appearance_fwd", "mmmot_pointnet_fwd", "mmmot_fusion_det_fwd", "mmmot_affinity_fwd",
              "mmmot_lp_assign"]

@@ -7,7 +7,7 @@ sys.path.insert(0, ROOT)
 from mmmot_b200 import _lib
 from mmmot_b200.weights import pack_tc
 lib = _lib.load()
-lib.mmmot_set_debug(int(os.environ.get('TC_DBG', '0')))
+_lib.check(lib.mmmot_set_debug(int(os.environ.get('TC_DBG', '0'))), "mmmot_set_debug")
 if os.environ.get('MMMOT_KSEG'): lib.mmmot_set_kseg(int(os.environ['MMMOT_KSEG']))
 vp = lambda t: ctypes.c_void_p(t.data_ptr())
 g = torch.Generator().manual_seed(0)
