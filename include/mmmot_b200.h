@@ -90,7 +90,7 @@ enum mmmot_weight_id {
   MMMOT_W_NE_W3 = 137, MMMOT_W_NE_B3 = 138,
   /* ---- tensor-core operands: the same matrices split into FP16 hi/lo and pre-tiled in the UMMA
      canonical K-major core-matrix layout  [k chunk 32][m tile 128][hi|lo][k group 4][m group 16][8][8]
-     (zero padded to multiples of 128 rows / 32 k); see csrc/gemm_tc.cuh.  VGG layer 0 (fp32 NCHW crops) uses
+     (zero padded to multiples of 128 rows / 32 k); see csrc/tc_common.cuh.  VGG layer 0 (fp32 NCHW crops) uses
      the K order k = ci*9 + (ky*3+kx); layers 1..12 (packed FP16 NHWC activations) use k = (ky*3+kx)*Cin + ci. */
   MMMOT_W_VGG_WP0 = 139,          /* .. +12 */
   MMMOT_W_PN_WP1 = 152,           /* .. +4 : PointNet trunk layers 1..5 */

@@ -11,9 +11,7 @@
 // next layer's producers).
 #include <algorithm>
 
-#include "norm_ops.cuh"
-#include "gemm_gen.cuh"
-#include "tc_ops.cuh"
+#include "engines.cuh"
 
 namespace {
 
@@ -327,9 +325,8 @@ extern "C" int mmmot_affinity_fwd(const mmmot_weights* wts, int affinity_op, int
   const int pm = use_tc ? 2 : 1;   // GroupNorm partials per column tile
   if (use_tc) {
     MM_TRY(transpose_f32(feats, w.fcl, 512, L, G, st));
-    feats_range_kernel<<<148, 256, 0, st>>>(feats, (long)G * 512 * L, affinity_op == MMMOT_AFF_MULTIPLY ? 255.9f : 65504.f,
-                                           ar.status());
-    MM_LAUNCH_CHECK();
+    MM_TRY(feats_range_check(feats, (long)G * 512 * L, affinity_op == MMMOT_AFF_MULTIPLY ? 255.9f : 65504.f, ar.status(),
+                             st));
     GemmP p = gemm_defaults();
     p.bias = W[MMMOT_W_AF_B01]; p.M = 1024; p.K = 512;
     p.S = NM; p.tiles_per_group = tpg; p.num_tiles = tpg * G;

@@ -164,7 +164,7 @@ extern "C" int mmmot_timing_collect(double* total_ms, double* total_flop, long* 
 
 // ---------------------------------------------------------------------------------------------
 // Engine selection + single-contraction test hook.
-#include "gemm_gen.cuh"
+#include "engines.cuh"
 
 namespace { int g_engine = 0; int g_dbg = 0; int g_kseg = 36; }
 int mm_kseg_chunks() { return g_kseg; }
@@ -221,7 +221,7 @@ extern "C" int mmmot_debug_linear_planar(const void* Wp, float wp_scale, const f
   p.bias = bias; p.M = M; p.K = K;
   p.S = (int)rows; p.tiles_per_group = mm_cdiv(rows, tc::BN); p.num_tiles = p.tiles_per_group;
   p.Y = Y; p.y_ms = M;
-  return gemm_tma_launch_mat(p, (const uint4*)Wp, wp_scale, (const __half*)Xhi, rows * (long)K, rows, K, tc::OUT_CL, 0,
+  return gemm_tma_launch_mat(p, (const uint4*)Wp, wp_scale, (const __half*)Xhi, rows * (long)K, rows, K,
                              (cudaStream_t)stream);
 }
 

@@ -2,7 +2,7 @@
 // Replaces reference modules/appear_net.py:166-190 (vgg_forward + SkipPool.forward :27-32).
 #include <cuda_fp16.h>
 
-#include "gemm_tma.cuh"
+#include "engines.cuh"
 
 namespace {
 
@@ -123,7 +123,7 @@ __global__ void __launch_bounds__(256) im2col27_kernel(const float* __restrict__
       for (int kx = 0; kx < 3; kx++) {
         const int yy = y + ky - 1, xx = x + kx - 1;
         const float v = (yy >= 0 && yy < H && xx >= 0 && xx < W) ? __ldg(src + (long)ci * hw + yy * W + xx) : 0.f;
-        tma::split_f16(v, h[ci * 9 + ky * 3 + kx], l[ci * 9 + ky * 3 + kx]);
+        split_f16(v, h[ci * 9 + ky * 3 + kx], l[ci * 9 + ky * 3 + kx]);
         amax = fmaxf(amax, fabsf(v));
       }
   mm_range_flag(status, amax);
@@ -259,9 +259,8 @@ extern "C" int mmmot_appearance_fwd(const mmmot_weights* wts, const float* crops
           p.bias = wts->w[MMMOT_W_VGG_B0]; p.M = cout; p.K = 32; p.relu = 1;
           p.S = (int)n_pix; p.tiles_per_group = mm_cdiv(n_pix, tc::BN); p.num_tiles = p.tiles_per_group;
           p.Y = reinterpret_cast<float*>(hb[which]); p.y_ms = cout;
-          MM_TRY(gemm_tma_launch_mat(p, (const uint4*)wts->w[MMMOT_W_VGG_WP0], wts->tc_scale[MMMOT_W_VGG_WP0], cols,
-                                     n_pix * 32, n_pix, 32, tma::OUT_PLANAR, plane_out, st, nullptr, status, nullptr,
-                                     (const uint4*)wts->w[MMMOT_W_VGG_WPX0]));
+          MM_TRY(gemm_tma_px_launch_mat(p, (const uint4*)wts->w[MMMOT_W_VGG_WPX0], wts->tc_scale[MMMOT_W_VGG_WP0], cols,
+                                        n_pix * 32, n_pix, 32, plane_out, status, st));
         }
       } else {
         GemmP p = gemm_defaults();

@@ -1,5 +1,6 @@
 // Shared helpers for libmmmot_sm100a.so (sm_100a only; no torch headers).
 #pragma once
+#include <cuda_fp16.h>
 #include <cuda_runtime.h>
 #include <stdint.h>
 #include <stdio.h>
@@ -103,3 +104,26 @@ __device__ __forceinline__ void mm_range_track2(uint32_t& acc, uint32_t hi2) {
 __device__ __forceinline__ void mm_range_flag2(int* status, uint32_t acc) {
   if (status && ((acc & 0xFFFFu) >= 0x7BFFu || (acc >> 16) >= 0x7BFFu)) atomicOr(status, 1);
 }
+
+// x -> FP16 hi/lo pair, x = hi + lo + O(2^-22 |x|), the operand format of the tcgen05 engines
+__device__ __forceinline__ void split_f16(float x, __half& hi, __half& lo) {
+  unsigned short a, b;
+  asm("{\n\t.reg .f32 f;\n\t"
+      "cvt.rn.satfinite.f16.f32 %0, %2;\n\t"
+      "cvt.f32.f16 f, %0;\n\t"
+      "sub.f32 f, %2, f;\n\t"
+      "cvt.rn.satfinite.f16.f32 %1, f;\n\t}"
+      : "=h"(a), "=h"(b)
+      : "f"(x));
+  hi = __ushort_as_half(a);
+  lo = __ushort_as_half(b);
+}
+__device__ __forceinline__ void split4_store(float4 x, __half* hi, __half* lo, int* status) {
+  mm_range_flag(status, fmaxf(fmaxf(fabsf(x.x), fabsf(x.y)), fmaxf(fabsf(x.z), fabsf(x.w))));
+  __half h[4], l[4];
+  split_f16(x.x, h[0], l[0]); split_f16(x.y, h[1], l[1]);
+  split_f16(x.z, h[2], l[2]); split_f16(x.w, h[3], l[3]);
+  *reinterpret_cast<uint2*>(hi) = *reinterpret_cast<uint2*>(h);
+  *reinterpret_cast<uint2*>(lo) = *reinterpret_cast<uint2*>(l);
+}
+

@@ -2,9 +2,7 @@
 // Replaces reference modules/fusion_net.py:31-42 (C), :62-70 (B), :85-92 (A) and
 // modules/tracking_net.py:149-163 (determine_det, eval) with w_det from :92-100.
 // GroupNorm(D,D) here normalises each channel over the L detections of one frame-pair.
-#include "gemm_simt.cuh"
-#include "norm_ops.cuh"
-#include "gemm_gen.cuh"
+#include "engines.cuh"
 
 namespace {
 

@@ -18,17 +18,15 @@
 // issuer, warp 9 weight loader (cp.async.bulk of pre-tiled FP16 hi/lo blocks), warps 10-17 operand producers.
 // One mbarrier per stage collects the loader's expect_tx and the eight producer warps' arrivals.
 #pragma once
-#include "gemm_tma.cuh"
+#include "tc_common.cuh"
 
 namespace gen {
 
 using namespace tc;
 
-enum { GEN_PAIR_MUL = 0, GEN_PAIR_ABS = 1, GEN_PAIR_SUB = 2, GEN_NORM = 3, GEN_COPY = 4 };   // GEN_PAIR_* == MMMOT_AFF_*
-
 constexpr int G_EPI_WARPS = 8, G_MMA_WARP = 8, G_LOAD_WARP = 9, G_PROD_WARP0 = 10, G_PROD_WARPS = 8;
 constexpr int G_THREADS = (G_PROD_WARP0 + G_PROD_WARPS) * 32;   // 576
-constexpr size_t G_SMEM_BYTES = (size_t)STAGES * STAGE_BYTES + 1024 + 256;
+constexpr size_t G_SMEM_BYTES = tc_smem_bytes(STAGE_BYTES);
 constexpr int G_MAX_K = 512;   // producer-side GroupNorm affine staged in shared memory
 
 struct GenP {
@@ -40,7 +38,7 @@ struct GenP {
   const float* gsh;
   int n, m, Lf;        // PAIR: columns s = i*m + j, objs = feature rows [0, n), dets = [n, n + m), Lf = n + m
   // FP16 range: the producers do not track the magnitudes they convert (their instruction stream is the kernel's
-  // bottleneck); the callers bound the operand instead — PAIR: feats_cl_check_kernel on the feature stacks, NORM:
+  // bottleneck); the callers bound the operand instead — PAIR: feats_range_kernel on the feature stacks, NORM:
   // gn_finalize's bound sqrt(count)*|gamma| + |beta| on the normalised values (both raise the status flag).
 };
 
@@ -62,53 +60,15 @@ static __global__ void __launch_bounds__(G_THREADS, 1) gemm_gen_kernel(const Gen
   const GemmP& p = P.t.g;
   extern __shared__ uint8_t smem_raw[];
   __shared__ __align__(16) float s_gsc[GEN == GEN_NORM ? G_MAX_K : 4], s_gsh[GEN == GEN_NORM ? G_MAX_K : 4];
-  const uint32_t raw = smem_u32(smem_raw);
-  const uint32_t base = (raw + 1023u) & ~1023u;
-  uint8_t* sm = smem_raw + (base - raw);
-  const uint32_t bar0 = base + STAGES * STAGE_BYTES;
-  auto full_bar = [&](int s) { return bar0 + 8u * s; };
-  auto empty_bar = [&](int s) { return bar0 + 8u * (STAGES + s); };
-  auto tfull_bar = [&](int b) { return bar0 + 8u * (2 * STAGES + b); };
-  auto tempty_bar = [&](int b) { return bar0 + 8u * (2 * STAGES + 2 + b); };
-  uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(sm + STAGES * STAGE_BYTES + 8 * (2 * STAGES + 4));
-
   const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
+  // full: the loader's expect_tx arrive + one arrive per producer warp
+  const TcPipe C = tc_begin<STAGE_BYTES>(smem_raw, 1 + G_PROD_WARPS, G_EPI_WARPS, warp == G_MMA_WARP);
+
   const int MT = P.t.mt_per_cta;
   const int mgroups = (P.t.m_tiles + MT - 1) / MT;
   const long total_tiles = (long)p.num_tiles * mgroups;
   const int KC = P.t.k_chunks;
   const int nbuf = (MT == 1) ? 2 : 1;   // accumulator buffers in TMEM (256 columns each when MT == 1)
-
-  if (tid == 0) {
-    for (int s = 0; s < STAGES; s++) {
-      mbar_init(full_bar(s), 1 + G_PROD_WARPS);   // loader's expect_tx arrive + one arrive per producer warp
-      mbar_init(empty_bar(s), 1);                 // tcgen05.commit
-    }
-    for (int b = 0; b < 2; b++) {
-      mbar_init(tfull_bar(b), 1);
-      mbar_init(tempty_bar(b), G_EPI_WARPS);
-    }
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-  }
-  if (warp == G_MMA_WARP) {
-    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(tmem_slot)),
-                 "r"(512)
-                 : "memory");
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
-  }
-  tc_fence_before();
-  __syncthreads();
-  tc_fence_after();
-  const uint32_t tmem_base = *tmem_slot;
-
-  // column tile -> group / first column / valid length
-  // (table tiling: {group, first ABSOLUTE row, length}; x_gs and y_gs are 0 then)
-  auto tile_cols = [&](int nt, int& g, int& c0, int& len) {
-    if (p.tile_tab) { const int4 tt = p.tile_tab[nt]; g = tt.x; c0 = tt.y; len = tt.z; return; }
-    g = nt / p.tiles_per_group;
-    c0 = (nt - g * p.tiles_per_group) * BN;
-    len = min(BN, p.S - c0);
-  };
 
   if (warp < G_EPI_WARPS) {
     // =============================== EPILOGUE ===============================
@@ -118,10 +78,9 @@ static __global__ void __launch_bounds__(G_THREADS, 1) gemm_gen_kernel(const Gen
       const int mg = (int)(t % mgroups);
       const int nt = (int)(t / mgroups);
       int g, c0, len;
-      tile_cols(nt, g, c0, len);
-      const int abuf = nbuf == 2 ? (int)(wcount & 1) : 0;
-      const uint32_t ause = nbuf == 2 ? (wcount >> 1) : wcount;
-      mbar_wait(tfull_bar(abuf), ause & 1);
+      tile_cols(p, nt, g, c0, len);
+      const int abuf = acc_buf(wcount, nbuf);
+      mbar_wait(C.tfull_bar(abuf), acc_parity(wcount, nbuf));
       tc_fence_after();
       for (int mt = 0; mt < MT; mt++) {
         const int co = (mg * MT + mt) * 128 + q * 32 + lane;
@@ -135,7 +94,7 @@ static __global__ void __launch_bounds__(G_THREADS, 1) gemm_gen_kernel(const Gen
           const int col0 = half * 128 + cc * 32;
           if (col0 >= len) break;   // warp-uniform
           uint32_t v[32];
-          tmem_ld32(tmem_base + ((uint32_t)(q * 32) << 16) + (uint32_t)(abuf * 256 + mt * 256 + col0), v);
+          tmem_ld32(C.tmem + ((uint32_t)(q * 32) << 16) + (uint32_t)(abuf * 256 + mt * 256 + col0), v);
           if (P.t.dbg & 1) continue;
           float s1 = 0.f, s2 = 0.f;
           if (col0 + 32 <= len) {
@@ -168,40 +127,27 @@ static __global__ void __launch_bounds__(G_THREADS, 1) gemm_gen_kernel(const Gen
       }
       tc_fence_before();
       __syncwarp();
-      if (lane == 0) mbar_arrive(tempty_bar(abuf));
+      if (lane == 0) mbar_arrive(C.tempty_bar(abuf));
     }
   } else if (warp == G_MMA_WARP) {
     // =============================== MMA ISSUER ===============================
     if (lane == 0) {
       uint32_t it = 0, tcount = 0;
       for (long t = blockIdx.x; t < total_tiles; t += gridDim.x, tcount++) {
-        const int abuf = nbuf == 2 ? (int)(tcount & 1) : 0;
-        const uint32_t ause = nbuf == 2 ? (tcount >> 1) : tcount;
-        mbar_wait(tempty_bar(abuf), (ause & 1) ^ 1);
+        const int abuf = acc_buf(tcount, nbuf);
+        mbar_wait(C.tempty_bar(abuf), acc_parity(tcount, nbuf) ^ 1);
         tc_fence_after();
         for (int kc = 0; kc < KC; kc++, it++) {
-          const int s = it % STAGES;
-          mbar_wait(full_bar(s), (it / STAGES) & 1);
+          const int s = ring_stage(it);
+          mbar_wait(C.full_bar(s), ring_parity(it));
           tc_fence_after();
-          const uint32_t sa = base + s * STAGE_BYTES, sb = sa + 2 * A_SUB;
+          const uint32_t sa = C.base + s * STAGE_BYTES, sb = sa + 2 * A_SUB;
 #pragma unroll
-          for (int mt = 0; mt < 2; mt++) {
-            if (mt < MT && !(P.t.dbg & 8)) {
-#pragma unroll
-              for (int ks = 0; ks < 2; ks++) {
-                const uint64_t a_hi = smem_desc(sa + mt * A_SUB + ks * 2 * A_LBO, A_LBO, SBO);
-                const uint64_t a_lo = smem_desc(sa + mt * A_SUB + A_HALF + ks * 2 * A_LBO, A_LBO, SBO);
-                const uint64_t b_hi = smem_desc(sb + ks * 2 * B_LBO, B_LBO, SBO);
-                const uint64_t b_lo = smem_desc(sb + B_HALF + ks * 2 * B_LBO, B_LBO, SBO);
-                const uint32_t d = tmem_base + (uint32_t)(abuf * 256 + mt * 256);
-                umma_f16(d, a_hi, b_hi, IDESC, (kc | ks) ? 1u : 0u);
-                umma_f16(d, a_hi, b_lo, IDESC, 1u);
-                umma_f16(d, a_lo, b_hi, IDESC, 1u);
-              }
-            }
-          }
-          umma_commit(empty_bar(s));                       // stage free once these MMAs have read it
-          if (kc == KC - 1) umma_commit(tfull_bar(abuf));  // accumulators complete
+          for (int mt = 0; mt < 2; mt++)
+            if (mt < MT && !(P.t.dbg & 8))
+              umma_hilo_chunk<false>(C.tmem + (uint32_t)(abuf * 256 + mt * 256), sa + mt * A_SUB, sb, kc);
+          umma_commit(C.empty_bar(s));                       // stage free once these MMAs have read it
+          if (kc == KC - 1) umma_commit(C.tfull_bar(abuf));  // accumulators complete
         }
       }
     }
@@ -215,13 +161,13 @@ static __global__ void __launch_bounds__(G_THREADS, 1) gemm_gen_kernel(const Gen
         const int mt0 = mg * MT;
         const int nmt = min(MT, P.t.m_tiles - mt0);
         for (int kc = 0; kc < KC; kc++, it++) {
-          const int s = it % STAGES;
-          mbar_wait(empty_bar(s), ((it / STAGES) & 1) ^ 1);
+          const int s = ring_stage(it);
+          mbar_wait(C.empty_bar(s), ring_parity(it) ^ 1);
           const uint32_t bytes = (uint32_t)nmt * A_SUB;
-          if (P.t.dbg & 2) { mbar_arrive(full_bar(s)); continue; }
-          mbar_expect_tx(full_bar(s), bytes);
+          if (P.t.dbg & 2) { mbar_arrive(C.full_bar(s)); continue; }
+          mbar_expect_tx(C.full_bar(s), bytes);
           const uint8_t* src = reinterpret_cast<const uint8_t*>(P.t.Wp) + ((size_t)kc * P.t.m_tiles + mt0) * A_SUB;
-          bulk_g2s(base + s * STAGE_BYTES, src, bytes, full_bar(s));
+          bulk_g2s(C.base + s * STAGE_BYTES, src, bytes, C.full_bar(s));
         }
       }
     }
@@ -249,7 +195,7 @@ static __global__ void __launch_bounds__(G_THREADS, 1) gemm_gen_kernel(const Gen
     for (long t = blockIdx.x; t < total_tiles; t += gridDim.x) {
       const int nt = (int)(t / mgroups);
       int g, c0, len;
-      tile_cols(nt, g, c0, len);
+      tile_cols(p, nt, g, c0, len);
       unsigned okmask = 0;
       // 32-bit element offsets of the items' rows (this thread's k group) relative to the tile's / group's base
       const float* tbase = ROWS ? P.src + ((long)g * p.x_gs + c0) * P.ld_src : P.src + (long)g * P.Lf * p.K;
@@ -291,9 +237,9 @@ static __global__ void __launch_bounds__(G_THREADS, 1) gemm_gen_kernel(const Gen
       };
       // wait for the ring slot, convert + store the chunk, publish it
       auto emit = [&](const Raw& R, int kc) {
-        const int s = it % STAGES;
-        mbar_wait(empty_bar(s), ((it / STAGES) & 1) ^ 1u);
-        uint8_t* bh = sm + s * STAGE_BYTES + 2 * A_SUB + off0;
+        const int s = ring_stage(it);
+        mbar_wait(C.empty_bar(s), ring_parity(it) ^ 1u);
+        uint8_t* bh = C.sm + s * STAGE_BYTES + 2 * A_SUB + off0;
         if (!(P.t.dbg & 4)) {
           const uint32_t sca = smem_u32(s_gsc + kc * BK + kg * 8), sha = smem_u32(s_gsh + kc * BK + kg * 8);
           float4 sc0, sc1, sh0, sh1;
@@ -330,7 +276,7 @@ static __global__ void __launch_bounds__(G_THREADS, 1) gemm_gen_kernel(const Gen
         }
         fence_async_smem();   // generic-proxy writes -> visible to the tensor core (async proxy)
         __syncwarp();
-        if (lane == 0) mbar_arrive(full_bar(s));
+        if (lane == 0) mbar_arrive(C.full_bar(s));
         it++;
       };
       if (PREFETCH) {
@@ -354,20 +300,11 @@ static __global__ void __launch_bounds__(G_THREADS, 1) gemm_gen_kernel(const Gen
     }
   }
 
-  // ---- teardown ----
-  tc_fence_before();
-  __syncthreads();
-  if (warp == G_MMA_WARP) {
-    asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(512) : "memory");
-  }
+  tc_end(C.tmem, warp == G_MMA_WARP);
 }
 
 }  // namespace gen
 
-// Host launcher.  g: M, K (multiple of 32, <= 512 for GEN_NORM), bias, S / tiles_per_group / num_tiles (uniform column
-// tiling, 256 columns per tile) or tile_tab (GEN_NORM: ragged groups, absolute rows), x_gs (NORM: source rows per group), Y / y_gs / y_ms = fp32 channels-last output (or
-// null), part = two GroupNorm partials per tile (stats_reduce(..., mult = 2)).  Wp = weights packed by
-// weights.py::pack_tc.  PAIR: src = fcl [G][Lf][K]; NORM: src = [G*x_gs][ld_src] fp32, gsc/gsh [G][K].
 template <int GEN, bool PAIRED>
 static int gemm_gen_launch_t(const GemmP& g, const uint4* Wp, float out_scale, const float* src, int ld_src,
                            const float* gsc, const float* gsh, int n, int m, int Lf, cudaStream_t st) {
@@ -375,33 +312,22 @@ static int gemm_gen_launch_t(const GemmP& g, const uint4* Wp, float out_scale, c
   if (g.tile_tab && ((GEN != gen::GEN_NORM && GEN != gen::GEN_COPY) || g.x_gs || g.y_gs)) return MMMOT_E_ARG;
   if (GEN == gen::GEN_NORM && (g.K > gen::G_MAX_K || !gsc || !gsh)) return MMMOT_E_ARG;
   if ((GEN == gen::GEN_NORM || GEN == gen::GEN_COPY) && (ld_src < g.K || (ld_src & 7))) return MMMOT_E_ARG;
-  int sms = 0;
-  MM_TRY(mm_sm_count(&sms));
-  static std::atomic<unsigned long long> attr{0};
-  MM_TRY(mm_ensure_smem(gen::gemm_gen_kernel<GEN, PAIRED>, gen::G_SMEM_BYTES, attr));
   gen::GenP P;
   memset(&P, 0, sizeof(P));
-  P.t.g = g;
-  P.t.Wp = Wp;
-  P.t.m_tiles = (g.M + 127) / 128;
-  P.t.k_chunks = g.K / tc::BK;
-  P.t.mt_per_cta = P.t.m_tiles >= 2 ? 2 : 1;   // M = 128: one subtile, two TMEM accumulator buffers
-  P.t.out_scale = out_scale;
-  P.t.out_mode = tc::OUT_CL;
-  P.t.dbg = mm_debug_flags();
+  P.t = tc::tc_params(g, Wp, out_scale, true);   // M = 128: one subtile, two TMEM accumulator buffers
   P.src = src; P.ld_src = ld_src; P.gsc = gsc; P.gsh = gsh;
   P.n = n; P.m = m; P.Lf = Lf;
-  const long mgroups = (P.t.m_tiles + P.t.mt_per_cta - 1) / P.t.mt_per_cta;
-  const long total = (long)g.num_tiles * mgroups;
-  const int grid = (int)(total < sms ? total : sms);
+  static std::atomic<unsigned long long> attr{0};
+  int grid = 0;
+  MM_TRY(tc::tc_grid(gen::gemm_gen_kernel<GEN, PAIRED>, gen::G_SMEM_BYTES, attr, P.t, &grid));
   gen::gemm_gen_kernel<GEN, PAIRED><<<grid, gen::G_THREADS, gen::G_SMEM_BYTES, st>>>(P);
   MM_LAUNCH_CHECK();
   return 0;
 }
 
 template <int GEN>
-static int gemm_gen_launch(const GemmP& g, const uint4* Wp, float out_scale, const float* src, int ld_src,
-                           const float* gsc, const float* gsh, int n, int m, int Lf, cudaStream_t st) {
+int gemm_gen_launch(const GemmP& g, const uint4* Wp, float out_scale, const float* src, int ld_src, const float* gsc,
+                    const float* gsh, int n, int m, int Lf, cudaStream_t st) {
   // PAIRED as documented at gemm_gen_kernel
   if constexpr (GEN == gen::GEN_NORM)
     return gemm_gen_launch_t<GEN, false>(g, Wp, out_scale, src, ld_src, gsc, gsh, n, m, Lf, st);

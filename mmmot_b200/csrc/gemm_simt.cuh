@@ -14,42 +14,7 @@
 // This is the accuracy-first engine (plain FP32 FFMA, 128x128x16 tiles, 8x8 register blocking).
 // fp32-exact operand arithmetic is what the 1e-4 parity bound needs (SURVEY F8).
 #pragma once
-#include "common.cuh"
-
-enum { XM_DIRECT = 0, XM_NORM_RELU = 1, XM_PAIR_MUL = 2, XM_PAIR_ABS = 3, XM_PAIR_SUB = 4, XM_CONV3 = 5 };
-
-struct GemmP {
-  // A operand: transposed weights Wt[K][ldw], output channels [m_base, m_base + M)
-  const float* Wt;
-  int ldw;
-  const float* bias;  // [M] or null
-  int M, K;
-  // column tiling: uniform (tile_tab == null): every group has S columns; else table of
-  // {group, first column (absolute), length, 0}
-  int S;
-  int tiles_per_group;
-  const int4* tile_tab;
-  int num_tiles;
-  // X operand: X + g*x_gs + k*x_ks + col   (col = column inside group for uniform tiling,
-  // absolute column for table tiling, where x_gs must be 0)
-  const float* X;
-  long x_gs, x_ks;
-  const float* sc;  // [G][K]
-  const float* sh;
-  // pair generator: F[g][K][Lf], objs = columns [0,n), dets = columns [n, n+m)
-  int n, m, Lf;
-  // conv3x3: X = in[img][Cin][H][W], Y = out[img][M][H][W]; S = n_img*H*W in one group
-  int H, W, Cin;
-  // output: Y + g*y_gs + co*y_ms + col ; null = statistics only
-  float* Y;
-  long y_gs, y_ms;
-  double2* part;        // [num_tiles][M] per-tile (sum, sumsq) partials or null; reduced in fixed
-                        // order by stats_reduce (no atomics: results are run-to-run bit-identical)
-  const float* addend;  // Y += addend[co*ld_add + seg[col]] or null
-  const int* seg;
-  int ld_add;
-  int relu;
-};
+#include "engines.cuh"
 
 template <int MODE, int TM>
 __global__ void __launch_bounds__(256, 2) gemm_simt_kernel(const GemmP p) {
@@ -283,9 +248,8 @@ __global__ void __launch_bounds__(256, 2) gemm_simt_kernel(const GemmP p) {
   }
 }
 
-// Host-side launcher.  p.M must be a multiple of 64.
 template <int MODE>
-static int gemm_simt_launch(const GemmP& p, cudaStream_t st) {
+int gemm_simt_launch(const GemmP& p, cudaStream_t st) {
   if (p.M % 64 != 0 || p.num_tiles <= 0) return MMMOT_E_SHAPE;
   if (p.M % 128 == 0) {
     gemm_simt_kernel<MODE, 128><<<(unsigned)((long)p.num_tiles * (p.M / 128)), 256, 0, st>>>(p);
@@ -294,10 +258,4 @@ static int gemm_simt_launch(const GemmP& p, cudaStream_t st) {
   }
   MM_LAUNCH_CHECK();
   return 0;
-}
-
-static inline GemmP gemm_defaults() {
-  GemmP p;
-  memset(&p, 0, sizeof(p));
-  return p;
 }

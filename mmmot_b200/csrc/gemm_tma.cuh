@@ -1,7 +1,7 @@
 // tcgen05 contraction engine, TMA-fed variant (sm_100a).
 //
-// Same arithmetic as gemm_tc.cuh (FP16 hi/lo split operands, 3 MMAs per k-step, FP32 accumulate in
-// TMEM, fused epilogue) but the generated operand is not produced by threads: activations between
+// Same arithmetic as the generated-operand kernel (gemm_gen.cuh: FP16 hi/lo split operands, 3 MMAs per k-step, FP32
+// accumulate in TMEM, fused epilogue) but the activation operand is not produced by threads: activations between
 // tensor-core layers live in HBM as two FP16 planes (hi, lo), channels-last, and the TMA engine
 // (cp.async.bulk.tensor, tiled mode, 64-byte swizzle) drops each [256 rows x 32 channels] box straight
 // into shared memory in the UMMA K-major SWIZZLE_64B layout:
@@ -14,6 +14,7 @@
 // When the tile has one 128-row subtile (Cout <= 128) the 512 TMEM columns hold TWO accumulator buffers, so
 // the epilogue of tile i overlaps the MMAs of tile i+1.  Conv outputs are transposed through a per-warp smem
 // scratch so each lane stores 64 contiguous bytes (32 channels of one pixel) per plane.
+// Compiled in engines.cu only: the launchers below have external linkage (see engines.cuh).
 #pragma once
 #include <cuda.h>
 #include <cuda_fp16.h>
@@ -26,33 +27,8 @@ using namespace tc;
 
 constexpr int T_THREADS = 320;
 constexpr int T_EPI_WARPS = 8, T_MMA_WARP = 8, T_LOAD_WARP = 9;
-constexpr int T_SCRATCH = 0;
 constexpr int T_EPI_SCRATCH = 32 * 80;   // per epilogue warp: 32 pixels x (64 B of channels + 16 B pad)
-constexpr size_t T_SMEM_BYTES = (size_t)STAGES * STAGE_BYTES + 1024 + 256 + T_EPI_WARPS * T_EPI_SCRATCH;
-
-enum { OUT_PLANAR = 3 };   // two FP16 planes Y_hi[row][y_ms], Y_lo = Y_hi + plane_elems (channels-last)
-
-struct TmaP {
-  TcP t;                    // .g: M, K, bias, relu, part, Y, y_ms, y_gs, S/tiles ...
-  int conv;                 // 0: rows x C matrix ; 1: 3x3 conv on [img][H][W][C]
-  int bx, by, bi;           // conv box (pixels): columns of a tile = (ii*by + yy)*bx + xx
-  int tiles_x, tiles_y;     // conv tile grid per image group
-  int n_img, H, W, C;       // conv geometry (C = input channels)
-  long plane_elems;         // output: distance (in fp16 elements) between the hi and lo planes
-  int ksegs, kc_per_seg;    // conv: K is accumulated in `ksegs` TMEM passes of kc_per_seg chunks whose fp32
-  float* acc_scratch;       // partial sums are combined in fp32 RN through acc_scratch[pixel][M] (see launcher)
-  int pool;                 // fused 2x2 max-pool in the conv epilogue (both kernels): the pooled map is written
-  unsigned long long* pool_sum;   // channel-major conv + pool: if set, the pooled values are also summed per (image, channel)
-                            // into pool_sum[img][M] as 2^-32 fixed point (SkipPool's global average, order-independent)
-  unsigned long long* segsum;   // matrix mode: if set, nothing is stored; relu(x*sc[g][co] + sh[g][co]) is summed per
-                            // detection (g.seg[column]) into segsum[det][M] as 2^-32 fixed point (order-independent)
-  int* status;              // workspace status word (FP16 range flag of the planar outputs) or null
-  const float* gen_src;     // pixel-major kernel, GEN27 variant: fp32 NCHW 3-channel crops [n_img][3][H][W]; the 27 (+5 zero)
-                            // taps of every pixel (k = ci*9 + ky*3 + kx) are built in shared memory by producer warps
-  const int4* chunk_tab;    // matrix mode with g.seg: per (column tile, half) the four 32-column chunks' descriptors
-                            // (first detection index << 1) | (chunk complete and inside ONE detection); see
-                            // seg_chunk_tab_kernel.  One uniform 16-byte load per subtile instead of a load + 12 shuffles.
-};
+constexpr size_t T_SMEM_BYTES = tc_smem_bytes(STAGE_BYTES) + T_EPI_WARPS * T_EPI_SCRATCH;
 
 // chunk descriptors of the table-tiled contractions over ragged per-detection columns (PointNet): tab[tile*2 + half]
 static __global__ void seg_chunk_tab_kernel(const int4* __restrict__ tiles, int num_tiles, const int* __restrict__ seg,
@@ -88,11 +64,6 @@ __device__ __forceinline__ void tma_load_4d(uint32_t dst, const CUtensorMap* map
       ::"r"(dst), "l"(reinterpret_cast<uint64_t>(map)), "r"(c0), "r"(c1), "r"(c2), "r"(c3), "r"(mbar)
       : "memory");
 }
-// K-major SWIZZLE_64B operand: rows of 64 bytes (32 fp16), 8-row groups 512 B apart (SBO), layout type 4.
-__device__ __forceinline__ uint64_t smem_desc_sw64(uint32_t saddr) {
-  return (uint64_t)((saddr & 0x3FFFFu) >> 4) | ((uint64_t)1 << 16) | ((uint64_t)(512 >> 4) << 32) | (1ull << 46) |
-         (4ull << 61);
-}
 // one 32-byte (whole sector) store; dst 32-byte aligned
 __device__ __forceinline__ void st_global_256(void* dst, const uint4& a, const uint4& b) {
   asm volatile("st.global.v8.b32 [%0], {%1, %2, %3, %4, %5, %6, %7, %8};" ::"l"(dst), "r"(a.x), "r"(a.y), "r"(a.z),
@@ -102,19 +73,6 @@ __device__ __forceinline__ void st_global_256(void* dst, const uint4& a, const u
 __device__ __forceinline__ void st_global_256(void* dst, const uint32_t* r) {
   st_global_256(dst, make_uint4(r[0], r[1], r[2], r[3]), make_uint4(r[4], r[5], r[6], r[7]));
 }
-__device__ __forceinline__ void split_f16(float x, __half& hi, __half& lo) {
-  unsigned short a, b;
-  asm("{\n\t.reg .f32 f;\n\t"
-      "cvt.rn.satfinite.f16.f32 %0, %2;\n\t"
-      "cvt.f32.f16 f, %0;\n\t"
-      "sub.f32 f, %2, f;\n\t"
-      "cvt.rn.satfinite.f16.f32 %1, f;\n\t}"
-      : "=h"(a), "=h"(b)
-      : "f"(x));
-  hi = __ushort_as_half(a);
-  lo = __ushort_as_half(b);
-}
-
 // 2x2 max-pool of one 32-column chunk held by a thread (one channel): the chunk is 32/BX box rows of BX pixels, so its
 // 16/BX row pairs hold BX/2 windows each: o[a*(BX/2) + b] = window (rows 2a, 2a+1; columns 2b, 2b+1).  BX <= 16.
 template <int BX>
@@ -132,18 +90,11 @@ static __global__ void __launch_bounds__(T_THREADS, 1)
 gemm_tma_kernel(const TmaP P, const __grid_constant__ CUtensorMap map_hi, const __grid_constant__ CUtensorMap map_lo) {
   const GemmP& p = P.t.g;
   extern __shared__ uint8_t smem_raw[];
-  const uint32_t raw = smem_u32(smem_raw);
-  const uint32_t base = (raw + 1023u) & ~1023u;
-  uint8_t* sm = smem_raw + (base - raw);
-  const uint32_t bar0 = base + STAGES * STAGE_BYTES;
-  auto full_bar = [&](int s) { return bar0 + 8u * s; };
-  auto empty_bar = [&](int s) { return bar0 + 8u * (STAGES + s); };
-  auto tfull_bar = [&](int b) { return bar0 + 8u * (2 * STAGES + b); };
-  auto tempty_bar = [&](int b) { return bar0 + 8u * (2 * STAGES + 2 + b); };
-  uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(sm + STAGES * STAGE_BYTES + 8 * (2 * STAGES + 4));
-  uint8_t* epi_scratch = sm + STAGES * STAGE_BYTES + 256;
-
   const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
+  // full: the loader's single expect_tx arrive (weights + 2 operand boxes)
+  const TcPipe C = tc_begin<STAGE_BYTES>(smem_raw, 1, T_EPI_WARPS, warp == T_MMA_WARP);
+  uint8_t* epi_scratch = C.sm + STAGES * STAGE_BYTES + 256;
+
   const int MT = P.t.mt_per_cta;
   const int mgroups = (P.t.m_tiles + MT - 1) / MT;
   const long total_tiles = (long)p.num_tiles * mgroups;
@@ -151,40 +102,6 @@ gemm_tma_kernel(const TmaP P, const __grid_constant__ CUtensorMap map_hi, const 
   const int KC = P.t.k_chunks;
   const int cchunks = P.conv ? P.C / BK : KC;
   const int nbuf = (MT == 1) ? 2 : 1;   // accumulator buffers in TMEM (256 columns each when MT == 1)
-
-  if (tid == 0) {
-    for (int s = 0; s < STAGES; s++) {
-      mbar_init(full_bar(s), 1);   // the loader's single expect_tx arrive (weights + 2 operand boxes)
-      mbar_init(empty_bar(s), 1);  // tcgen05.commit
-    }
-    for (int b = 0; b < 2; b++) {
-      mbar_init(tfull_bar(b), 1);
-      mbar_init(tempty_bar(b), T_EPI_WARPS);
-    }
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-  }
-  if (warp == T_MMA_WARP) {
-    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(tmem_slot)),
-                 "r"(512)
-                 : "memory");
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
-  }
-  tc_fence_before();
-  __syncthreads();
-  tc_fence_after();
-  const uint32_t tmem_base = *tmem_slot;
-
-  // tile -> (m group, column tile) ; column tile -> group / first column (matrix) or box origin (conv)
-  auto tile_cols = [&](int nt, int& g, int& c0, int& len) {
-    if (p.tile_tab) { int4 tt = p.tile_tab[nt]; g = tt.x; c0 = tt.y; len = tt.z; }
-    else { g = nt / p.tiles_per_group; c0 = (nt - g * p.tiles_per_group) * BN; len = min(BN, p.S - c0); }
-  };
-  auto conv_origin = [&](int nt, int& i0, int& y0, int& x0) {
-    const int tx = nt % P.tiles_x;
-    const int r = nt / P.tiles_x;
-    const int ty = r % P.tiles_y;
-    i0 = (r / P.tiles_y) * P.bi; y0 = ty * P.by; x0 = tx * P.bx;
-  };
 
   if (warp < T_EPI_WARPS) {
     // =============================== EPILOGUE ===============================
@@ -241,7 +158,7 @@ gemm_tma_kernel(const TmaP P, const __grid_constant__ CUtensorMap map_hi, const 
       psum = 0.f; psum_img = -1;
     };
     // o[q], q < NP: pooled pixels of box rows (r0, r0 + 1), columns 2q', in box-row units r = ii*by + yy
-    auto pool_emit = [&](const float (&o)[16], int np, int r0, int rstep_q, int wq, int cb, int co_, int i0, int y0, int x0) {
+    auto pool_emit = [&](const float (&o)[16], int np, int r0, int wq, int cb, int co_, int i0, int y0, int x0) {
       // pooled pixel q: box row r0 + 2*(q / wq), box column 2*(q % wq)      (wq = windows per row pair)
       float xs[32];
 #pragma unroll
@@ -253,7 +170,6 @@ gemm_tma_kernel(const TmaP P, const __grid_constant__ CUtensorMap map_hi, const 
       const bool ok = lane < np && img < P.n_img && y < P.H && xg < P.W;
       store_rows(xs, ok, (((long)img * Hp + (y >> 1)) * Wp + (xg >> 1)) * p.y_ms + cb);
       if (P.pool_sum) {
-        (void)rstep_q;
 #pragma unroll
         for (int j = 0; j < 16; j++) {
           if (j < np) {
@@ -279,7 +195,7 @@ gemm_tma_kernel(const TmaP P, const __grid_constant__ CUtensorMap map_hi, const 
         }
 #pragma unroll
         for (int b = 0; b < 16; b++) o[b] = fmaxf(hprev[b], fmaxf(x[2 * b], x[2 * b + 1]));
-        pool_emit(o, 16, r0 - 1, 0, 16, co_ - lane, co_, i0, y0, x0);
+        pool_emit(o, 16, r0 - 1, 16, co_ - lane, co_, i0, y0, x0);
         return;
       }
       float o8[8];
@@ -289,19 +205,18 @@ gemm_tma_kernel(const TmaP P, const __grid_constant__ CUtensorMap map_hi, const 
       else pool_chunk<2>(x, o8);
 #pragma unroll
       for (int j = 0; j < 16; j++) o[j] = j < 8 ? o8[j] : 0.f;
-      pool_emit(o, 8, r0, 0, P.bx >> 1, co_ - lane, co_, i0, y0, x0);
+      pool_emit(o, 8, r0, P.bx >> 1, co_ - lane, co_, i0, y0, x0);
     };
 
     for (long t = blockIdx.x; t < total_tiles; t += gridDim.x) {
       const int mg = (int)(t % mgroups);
       const int nt = (int)(t / mgroups);
       int g = 0, c0 = 0, len = BN, i0 = 0, y0 = 0, x0 = 0;
-      if (P.conv) conv_origin(nt, i0, y0, x0); else tile_cols(nt, g, c0, len);
+      if (P.conv) conv_origin(P, nt, i0, y0, x0); else tile_cols(p, nt, g, c0, len);
       for (int seg = 0; seg < P.ksegs; seg++, wcount++) {
-      const int abuf = nbuf == 2 ? (int)(wcount & 1) : 0;
-      const uint32_t ause = nbuf == 2 ? (wcount >> 1) : wcount;
+      const int abuf = acc_buf(wcount, nbuf);
       const uint32_t acc_col = (uint32_t)(abuf * 256);
-      mbar_wait(tfull_bar(abuf), ause & 1);
+      mbar_wait(C.tfull_bar(abuf), acc_parity(wcount, nbuf));
       tc_fence_after();
       if (P.ksegs > 1) {
         // K-segmented convolution: the tensor core's fp32 accumulator rounds toward zero at every K=16 step,
@@ -314,7 +229,7 @@ gemm_tma_kernel(const TmaP P, const __grid_constant__ CUtensorMap map_hi, const 
           for (int cc = 0; cc < 4; cc++) {
             const int col0 = half * 128 + cc * 32;
             uint32_t v[32];
-            tmem_ld32(tmem_base + ((uint32_t)(q * 32) << 16) + acc_col + (uint32_t)(mt * 256 + col0), v);
+            tmem_ld32(C.tmem + ((uint32_t)(q * 32) << 16) + acc_col + (uint32_t)(mt * 256 + col0), v);
             if (!rowok) continue;
             // partial sums live in TILE order, scratch[(tile*256 + column)][M]: no pixel arithmetic, and a
             // warp's 32 channels of one column are one 128-byte access
@@ -378,7 +293,7 @@ gemm_tma_kernel(const TmaP P, const __grid_constant__ CUtensorMap map_hi, const 
           const float adc = cc == 0 ? adv[0] : cc == 1 ? adv[1] : cc == 2 ? adv[2] : adv[3];
           const bool single = (one_det >> cc) & 1u;
           uint32_t v[32];
-          tmem_ld32(tmem_base + ((uint32_t)(q * 32) << 16) + acc_col + (uint32_t)(mt * 256 + col0), v);
+          tmem_ld32(C.tmem + ((uint32_t)(q * 32) << 16) + acc_col + (uint32_t)(mt * 256 + col0), v);
           if (P.t.dbg & 1) continue;
           float s1 = 0.f, s2 = 0.f;
           bool fast = col0 + 32 <= len;
@@ -453,35 +368,17 @@ gemm_tma_kernel(const TmaP P, const __grid_constant__ CUtensorMap map_hi, const 
 #pragma unroll
             for (int j = 0; j < 32; j++) xv[j] = __uint_as_float(v[j]);
             emit_conv(xv, cc, col0, co, i0, y0, x0);
-          } else {
+          } else {   // fp32 channels-last
             const int nvalid = min(32, len - col0);
             const long row0 = (long)g * p.y_gs + c0 + col0;
-            if (P.t.out_mode == OUT_PLANAR && !(p.y_ms & 31)) {
-              float xv[32];
+            float* dst = p.Y + row0 * p.y_ms + co;
+            if (nvalid == 32) {
 #pragma unroll
-              for (int j = 0; j < 32; j++) xv[j] = __uint_as_float(v[j]);
-              store_rows(xv, lane < nvalid, (row0 + lane) * p.y_ms + (co - lane));
-            } else if (P.t.out_mode == OUT_PLANAR) {
-              __half* dst = yh + row0 * p.y_ms + co;
+              for (int j = 0; j < 32; j++) { *dst = __uint_as_float(v[j]); dst += p.y_ms; }
+            } else {
 #pragma unroll
               for (int j = 0; j < 32; j++)
-                if (j < nvalid) {
-                  __half h, l;
-                  split_f16(__uint_as_float(v[j]), h, l);
-                  amax = fmaxf(amax, fabsf(__uint_as_float(v[j])));
-                  dst[(long)j * p.y_ms] = h;
-                  dst[(long)j * p.y_ms + P.plane_elems] = l;
-                }
-            } else {   // OUT_CL fp32 channels-last
-              float* dst = p.Y + row0 * p.y_ms + co;
-              if (nvalid == 32) {
-#pragma unroll
-                for (int j = 0; j < 32; j++) { *dst = __uint_as_float(v[j]); dst += p.y_ms; }
-              } else {
-#pragma unroll
-                for (int j = 0; j < 32; j++)
-                  if (j < nvalid) dst[(long)j * p.y_ms] = __uint_as_float(v[j]);
-              }
+                if (j < nvalid) dst[(long)j * p.y_ms] = __uint_as_float(v[j]);
             }
           }
         }
@@ -490,7 +387,7 @@ gemm_tma_kernel(const TmaP P, const __grid_constant__ CUtensorMap map_hi, const 
       }
       tc_fence_before();
       __syncwarp();
-      if (lane == 0) mbar_arrive(tempty_bar(abuf));
+      if (lane == 0) mbar_arrive(C.tempty_bar(abuf));
       }
     }
     mm_range_flag(P.status, amax);
@@ -500,34 +397,21 @@ gemm_tma_kernel(const TmaP P, const __grid_constant__ CUtensorMap map_hi, const 
       uint32_t it = 0, tcount = 0;
       for (long t = blockIdx.x; t < total_tiles; t += gridDim.x) {
        for (int seg = 0; seg < P.ksegs; seg++, tcount++) {
-        const int abuf = nbuf == 2 ? (int)(tcount & 1) : 0;
-        const uint32_t ause = nbuf == 2 ? (tcount >> 1) : tcount;
-        mbar_wait(tempty_bar(abuf), (ause & 1) ^ 1);
+        const int abuf = acc_buf(tcount, nbuf);
+        mbar_wait(C.tempty_bar(abuf), acc_parity(tcount, nbuf) ^ 1);
         tc_fence_after();
         const int kc_lo = seg * P.kc_per_seg, kc_hi = min(KC, kc_lo + P.kc_per_seg);
         for (int kc = kc_lo; kc < kc_hi; kc++, it++) {
-          const int s = it % STAGES;
-          mbar_wait(full_bar(s), (it / STAGES) & 1);
+          const int s = ring_stage(it);
+          mbar_wait(C.full_bar(s), ring_parity(it));
           tc_fence_after();
-          const uint32_t sa = base + s * STAGE_BYTES, sb = sa + 2 * A_SUB;
+          const uint32_t sa = C.base + s * STAGE_BYTES, sb = sa + 2 * A_SUB;
 #pragma unroll
-          for (int mt = 0; mt < 2; mt++) {
-            if (mt < MT && !(P.t.dbg & 8)) {
-#pragma unroll
-              for (int ks = 0; ks < 2; ks++) {
-                const uint64_t a_hi = smem_desc(sa + mt * A_SUB + ks * 2 * A_LBO, A_LBO, SBO);
-                const uint64_t a_lo = smem_desc(sa + mt * A_SUB + A_HALF + ks * 2 * A_LBO, A_LBO, SBO);
-                const uint64_t b_hi = smem_desc_sw64(sb + ks * 32);
-                const uint64_t b_lo = smem_desc_sw64(sb + B_HALF + ks * 32);
-                const uint32_t d = tmem_base + (uint32_t)(abuf * 256 + mt * 256);
-                umma_f16(d, a_hi, b_hi, IDESC, ((kc - kc_lo) | ks) ? 1u : 0u);
-                umma_f16(d, a_hi, b_lo, IDESC, 1u);
-                umma_f16(d, a_lo, b_hi, IDESC, 1u);
-              }
-            }
-          }
-          umma_commit(empty_bar(s));
-          if (kc == kc_hi - 1) umma_commit(tfull_bar(abuf));
+          for (int mt = 0; mt < 2; mt++)
+            if (mt < MT && !(P.t.dbg & 8))
+              umma_hilo_chunk<true>(C.tmem + (uint32_t)(abuf * 256 + mt * 256), sa + mt * A_SUB, sb, kc - kc_lo);
+          umma_commit(C.empty_bar(s));
+          if (kc == kc_hi - 1) umma_commit(C.tfull_bar(abuf));
         }
        }
       }
@@ -543,38 +427,33 @@ gemm_tma_kernel(const TmaP P, const __grid_constant__ CUtensorMap map_hi, const 
         const int mt0 = mg * MT;
         const int nmt = min(MT, P.t.m_tiles - mt0);
         int g = 0, c0 = 0, len = BN, i0 = 0, y0 = 0, x0 = 0;
-        if (P.conv) conv_origin(nt, i0, y0, x0); else tile_cols(nt, g, c0, len);
+        if (P.conv) conv_origin(P, nt, i0, y0, x0); else tile_cols(p, nt, g, c0, len);
         const int row0 = (int)((long)g * p.x_gs + c0);
         for (int kc = 0; kc < KC; kc++, it++) {
-          const int s = it % STAGES;
-          mbar_wait(empty_bar(s), ((it / STAGES) & 1) ^ 1);
+          const int s = ring_stage(it);
+          mbar_wait(C.empty_bar(s), ring_parity(it) ^ 1);
           const uint32_t abytes = (uint32_t)nmt * A_SUB;
           const bool skipA = P.t.dbg & 2, skipB = P.t.dbg & 4;     // profiling experiments only
-          mbar_expect_tx(full_bar(s), (skipA ? 0u : abytes) + (skipB ? 0u : 2u * B_HALF));
-          const uint32_t sa = base + s * STAGE_BYTES, sb = sa + 2 * A_SUB;
+          mbar_expect_tx(C.full_bar(s), (skipA ? 0u : abytes) + (skipB ? 0u : 2u * B_HALF));
+          const uint32_t sa = C.base + s * STAGE_BYTES, sb = sa + 2 * A_SUB;
           const uint8_t* src = reinterpret_cast<const uint8_t*>(P.t.Wp) + ((size_t)kc * P.t.m_tiles + mt0) * A_SUB;
-          if (!skipA) bulk_g2s(sa, src, abytes, full_bar(s));
+          if (!skipA) bulk_g2s(sa, src, abytes, C.full_bar(s));
           if (skipB) continue;
           if (P.conv) {
             const int tap = kc / cchunks, cc = kc - tap * cchunks;
             const int dx = tap % 3 - 1, dy = tap / 3 - 1;
-            tma_load_4d(sb, &map_hi, cc * BK, x0 + dx, y0 + dy, i0, full_bar(s));
-            tma_load_4d(sb + B_HALF, &map_lo, cc * BK, x0 + dx, y0 + dy, i0, full_bar(s));
+            tma_load_4d(sb, &map_hi, cc * BK, x0 + dx, y0 + dy, i0, C.full_bar(s));
+            tma_load_4d(sb + B_HALF, &map_lo, cc * BK, x0 + dx, y0 + dy, i0, C.full_bar(s));
           } else {
-            tma_load_2d(sb, &map_hi, kc * BK, row0, full_bar(s));
-            tma_load_2d(sb + B_HALF, &map_lo, kc * BK, row0, full_bar(s));
+            tma_load_2d(sb, &map_hi, kc * BK, row0, C.full_bar(s));
+            tma_load_2d(sb + B_HALF, &map_lo, kc * BK, row0, C.full_bar(s));
           }
         }
       }
     }
     __syncwarp();
   }
-
-  tc_fence_before();
-  __syncthreads();
-  if (warp == T_MMA_WARP) {
-    asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(512) : "memory");
-  }
+  tc_end(*C.tmem_slot(), warp == T_MMA_WARP);
 }
 
 // ---- host side: tensor maps through the driver entry point (no libcuda link dependency) ----
@@ -622,122 +501,104 @@ static inline int make_map_4d(CUtensorMap* m, const void* basep, int n_img, int 
 
 #include "gemm_tma_px.cuh"
 
-// pixel-major kernel for 64-channel planar outputs (see gemm_tma_px.cuh); P fully prepared by the caller, P.t.Wp = the
-// compact N = 64 weight tiles (weights.py::pack_px)
-static int gemm_tma_px_launch(tma::TmaP& P, const CUtensorMap& mh, const CUtensorMap& ml, int sms, cudaStream_t st) {
+int seg_chunk_tab(const int4* tiles, int num_tiles, const int* seg, int4* tab, cudaStream_t st) {
+  tma::seg_chunk_tab_kernel<<<mm_cdiv((long)num_tiles * 2, 128), 128, 0, st>>>(tiles, num_tiles, seg, tab);
+  MM_LAUNCH_CHECK();
+  return 0;
+}
+
+// P fully prepared by the caller
+static int gemm_tma_launch(const tc::TmaP& P, const CUtensorMap& mh, const CUtensorMap& ml, cudaStream_t st) {
   static std::atomic<unsigned long long> attr{0};
-  MM_TRY(mm_ensure_smem(tma::gemm_tma_px_kernel<false>, tma::PX_SMEM_BYTES, attr));
-  const long total = P.t.g.num_tiles;
-  const int grid = (int)(total < sms ? total : sms);
+  int grid = 0;
+  MM_TRY(tc::tc_grid(tma::gemm_tma_kernel, tma::T_SMEM_BYTES, attr, P.t, &grid));
+  tma::gemm_tma_kernel<<<grid, tma::T_THREADS, tma::T_SMEM_BYTES, st>>>(P, mh, ml);
+  MM_LAUNCH_CHECK();
+  return 0;
+}
+// pixel-major kernel for 64-channel planar outputs (see gemm_tma_px.cuh); P fully prepared by the caller, P.t.Wp = the
+// compact N = 64 weight tiles (weights.py::pack_px).  M = 64, so P.t.m_tiles = 1 and tc_grid's work items are the tiles.
+static int gemm_tma_px_launch(const tc::TmaP& P, const CUtensorMap& mh, const CUtensorMap& ml, cudaStream_t st) {
+  if (P.t.m_tiles != 1) return MMMOT_E_ARG;
+  static std::atomic<unsigned long long> attr{0};
+  int grid = 0;
+  MM_TRY(tc::tc_grid(tma::gemm_tma_px_kernel<false>, tma::PX_SMEM_BYTES, attr, P.t, &grid));
   tma::gemm_tma_px_kernel<false><<<grid, tma::T_THREADS, tma::PX_SMEM_BYTES, st>>>(P, mh, ml);
   MM_LAUNCH_CHECK();
   return 0;
 }
 
-// First VGG layer (3 -> 64 channels, 3x3 / pad 1) straight from the fp32 NCHW crops: the K = 32 operand (27 taps + 5
-// zeros per pixel, FP16 hi/lo) is generated in shared memory by the kernel's producer warps, so the im2col matrix
-// (128 B per pixel written and read back) never exists.  Output: planar FP16 NHWC, bias + ReLU applied.
-// Crop shapes it takes: a tile = 256 consecutive pixels of one image, and the tile's neighbourhood, (256 + 2W + 2) x 3
-// floats, is staged in two 8 KB weight slots.  Wider crops need the im2col27 pre-pass.
+// Crop shapes the GEN27 variant takes: a tile = 256 consecutive pixels of one image, and the tile's neighbourhood,
+// (256 + 2W + 2) x 3 floats, is staged in two 8 KB weight slots.  Wider crops need the im2col27 pre-pass.  The K = 32
+// operand (27 taps + 5 zeros per pixel, FP16 hi/lo) is generated in shared memory by the kernel's producer warps, so the
+// im2col matrix (128 B per pixel written and read back) never exists.  Output: planar FP16 NHWC, bias + ReLU applied.
 constexpr int PX_GEN27_MAX_W = 512;
 static_assert((tc::BN + 2 * PX_GEN27_MAX_W + 2) * 12 <= 2 * tma::PX_W_SLOT, "GEN27 staging buffer");
-static inline bool gemm_tma_px_gen27_fits(int H, int W) { return ((long)H * W) % tc::BN == 0 && W <= PX_GEN27_MAX_W; }
+bool gemm_tma_px_gen27_fits(int H, int W) { return ((long)H * W) % tc::BN == 0 && W <= PX_GEN27_MAX_W; }
 
-static int gemm_tma_px_launch_gen27(const float* crops, int n_img, int H, int W, const uint4* Wpx, float out_scale,
-                                    const float* bias, __half* Yhi, long y_plane, int* status, cudaStream_t st) {
+int gemm_tma_px_launch_gen27(const float* crops, int n_img, int H, int W, const uint4* Wpx, float out_scale,
+                             const float* bias, __half* Yhi, long y_plane, int* status, cudaStream_t st) {
   if (!crops || !Wpx || !Yhi) return MMMOT_E_ARG;
   const long n_pix = (long)n_img * H * W;
   if (n_pix >= (1L << 31) || !gemm_tma_px_gen27_fits(H, W)) return MMMOT_E_SHAPE;
-  int sms = 0;
-  MM_TRY(mm_sm_count(&sms));
-  static std::atomic<unsigned long long> attr{0};
-  MM_TRY(mm_ensure_smem(tma::gemm_tma_px_kernel<true>, tma::PX_SMEM_BYTES, attr));
-  tma::TmaP P;
+  tc::TmaP P;
   memset(&P, 0, sizeof(P));
   GemmP g = gemm_defaults();
   g.bias = bias; g.M = 64; g.K = 32; g.relu = 1;
   g.S = (int)n_pix; g.tiles_per_group = mm_cdiv(n_pix, tc::BN); g.num_tiles = g.tiles_per_group;
   g.Y = reinterpret_cast<float*>(Yhi); g.y_ms = 64;
-  P.t.g = g;
-  P.t.Wp = Wpx;
-  P.t.m_tiles = 1; P.t.k_chunks = 1; P.t.mt_per_cta = 1;
-  P.t.out_scale = out_scale;
-  P.t.out_mode = tma::OUT_PLANAR;
-  P.t.dbg = mm_debug_flags();
+  P.t = tc::tc_params(g, Wpx, out_scale, false);
   P.plane_elems = y_plane;
-  P.ksegs = 1; P.kc_per_seg = 1;
   P.status = status;
   P.gen_src = crops; P.n_img = n_img; P.H = H; P.W = W;
+  static std::atomic<unsigned long long> attr{0};
+  int grid = 0;
+  MM_TRY(tc::tc_grid(tma::gemm_tma_px_kernel<true>, tma::PX_SMEM_BYTES, attr, P.t, &grid));
   alignas(64) CUtensorMap dummy;
   memset(&dummy, 0, sizeof(dummy));
-  const long total = g.num_tiles;
-  const int grid = (int)(total < sms ? total : sms);
   tma::gemm_tma_px_kernel<true><<<grid, tma::PX_GEN_THREADS, tma::PX_SMEM_BYTES, st>>>(P, dummy, dummy);
   MM_LAUNCH_CHECK();
   return 0;
 }
 
-// 1x1 contraction on planar FP16 (hi, lo) channels-last activations X_hi[rows][ldx], X_lo = X_hi + x_plane.
-// g: M, K (multiple of 32), bias, tiles, x_gs (rows per group), Y / y_ms / y_gs, part, addend...
-// Wpx: the same weights as compact N = 64 tiles (weights.py::pack_px); given those, a plain 64-channel planar output
-// runs on the pixel-major kernel.
-static int gemm_tma_launch_mat(const GemmP& g, const uint4* Wp, float out_scale, const __half* Xhi, long x_plane,
-                               long rows, int ldx, int out_mode, long y_plane, cudaStream_t st,
-                               unsigned long long* segsum = nullptr, int* status = nullptr, const int4* chunk_tab = nullptr,
-                               const uint4* Wpx = nullptr) {
-  if (!Wp || g.num_tiles <= 0 || g.K % tc::BK) return MMMOT_E_ARG;
-  int sms = 0;
-  MM_TRY(mm_sm_count(&sms));
-  static std::atomic<unsigned long long> attr{0};
-  MM_TRY(mm_ensure_smem(tma::gemm_tma_kernel, tma::T_SMEM_BYTES, attr));
-  tma::TmaP P;
+int gemm_tma_px_launch_mat(const GemmP& g, const uint4* Wpx, float out_scale, const __half* Xhi, long x_plane, long rows,
+                           int ldx, long y_plane, int* status, cudaStream_t st) {
+  if (!Wpx || g.num_tiles <= 0 || g.K % tc::BK || g.M != 64 || g.y_ms != 64) return MMMOT_E_ARG;
+  tc::TmaP P;
   memset(&P, 0, sizeof(P));
-  P.t.g = g;
-  P.t.Wp = Wp;
-  P.t.m_tiles = (g.M + 127) / 128;
-  P.t.k_chunks = g.K / tc::BK;
-  // two 128-row subtiles per CTA share each operand box; short K chains (<= 16 chunks) are epilogue-bound instead,
-  // so they run one subtile per tile and double-buffer the accumulator in TMEM (epilogue overlaps the next MMAs).
-  // The arithmetic of a subtile does not depend on this choice.
-  P.t.mt_per_cta = (P.t.m_tiles >= 2 && P.t.k_chunks > 16) ? 2 : 1;
-  P.t.out_scale = out_scale;
-  P.t.out_mode = out_mode;
-  P.t.dbg = mm_debug_flags();
+  P.t = tc::tc_params(g, Wpx, out_scale, false);
   P.plane_elems = y_plane;
-  P.ksegs = 1; P.kc_per_seg = P.t.k_chunks;
-  P.segsum = segsum;
   P.status = status;
-  P.chunk_tab = chunk_tab;
-  if (g.seg && (g.addend || segsum) && !chunk_tab) return MMMOT_E_ARG;
   alignas(64) CUtensorMap mh, ml;
   MM_TRY(tma::make_map_2d(&mh, Xhi, rows, g.K, ldx));
   MM_TRY(tma::make_map_2d(&ml, Xhi + x_plane, rows, g.K, ldx));
-  if (Wpx && out_mode == tma::OUT_PLANAR && g.M == 64 && g.y_ms == 64 && !g.part && !segsum && !g.addend && !g.tile_tab) {
-    P.t.Wp = Wpx;
-    return gemm_tma_px_launch(P, mh, ml, sms, st);
-  }
-  const long mgroups = (P.t.m_tiles + P.t.mt_per_cta - 1) / P.t.mt_per_cta;
-  const long total = (long)g.num_tiles * mgroups;
-  const int grid = (int)(total < sms ? total : sms);
-  tma::gemm_tma_kernel<<<grid, tma::T_THREADS, tma::T_SMEM_BYTES, st>>>(P, mh, ml);
-  MM_LAUNCH_CHECK();
-  return 0;
+  return gemm_tma_px_launch(P, mh, ml, st);
 }
 
-// 3x3 / pad 1 convolution on planar FP16 NHWC activations; output planar FP16 NHWC (ReLU via g.relu).
-// acc_scratch (fp32 [tiles*256][M], tiles = ceil(W/bx)*ceil(H/by)*ceil(n/bi) <= padded pixel count) enables K-segmentation: chains longer than mmmot_set_kseg() chunks of 32 are
-// accumulated in several TMEM passes and summed in fp32 RN, which bounds the tensor core's round-toward-zero
-// accumulation error (DESIGN.md §4.2).  nullptr = single pass.
-static int gemm_tma_launch_conv(const GemmP& g0, const uint4* Wp, float out_scale, const __half* Xhi, long x_plane,
-                                int n_img, int H, int W, int C, __half* Yhi, long y_plane, cudaStream_t st,
-                                float* acc_scratch = nullptr, long y_plane_pooled = 0, int* did_pool = nullptr,
-                                int* status = nullptr, unsigned long long* pool_sum = nullptr, const uint4* Wpx = nullptr) {
+int gemm_tma_launch_mat(const GemmP& g, const uint4* Wp, float out_scale, const __half* Xhi, long x_plane, long rows,
+                        int ldx, cudaStream_t st, unsigned long long* segsum, const int4* chunk_tab) {
+  if (!Wp || g.num_tiles <= 0 || g.K % tc::BK) return MMMOT_E_ARG;
+  if (g.seg && (g.addend || segsum) && !chunk_tab) return MMMOT_E_ARG;
+  tc::TmaP P;
+  memset(&P, 0, sizeof(P));
+  // two 128-row subtiles per CTA share each operand box; short K chains (<= 16 chunks) are epilogue-bound instead,
+  // so they run one subtile per tile and double-buffer the accumulator in TMEM (epilogue overlaps the next MMAs).
+  // The arithmetic of a subtile does not depend on this choice.
+  P.t = tc::tc_params(g, Wp, out_scale, g.K / tc::BK > 16);
+  P.ksegs = 1; P.kc_per_seg = P.t.k_chunks;
+  P.segsum = segsum;
+  P.chunk_tab = chunk_tab;
+  alignas(64) CUtensorMap mh, ml;
+  MM_TRY(tma::make_map_2d(&mh, Xhi, rows, g.K, ldx));
+  MM_TRY(tma::make_map_2d(&ml, Xhi + x_plane, rows, g.K, ldx));
+  return gemm_tma_launch(P, mh, ml, st);
+}
+
+int gemm_tma_launch_conv(const GemmP& g0, const uint4* Wp, float out_scale, const __half* Xhi, long x_plane, int n_img,
+                         int H, int W, int C, __half* Yhi, long y_plane, cudaStream_t st, float* acc_scratch,
+                         long y_plane_pooled, int* did_pool, int* status, unsigned long long* pool_sum, const uint4* Wpx) {
   if (did_pool) *did_pool = 0;
   if (!Wp || C % tc::BK) return MMMOT_E_ARG;
-  int sms = 0;
-  MM_TRY(mm_sm_count(&sms));
-  static std::atomic<unsigned long long> attr{0};
-  MM_TRY(mm_ensure_smem(tma::gemm_tma_kernel, tma::T_SMEM_BYTES, attr));
   // box of 256 pixels = bx * by * bi (powers of two): the shape with the least padding waste, widest first
   int bx = 1, by = 1, bi = 256;
   {
@@ -760,7 +621,7 @@ static int gemm_tma_launch_conv(const GemmP& g0, const uint4* Wp, float out_scal
     px = w16 <= best + 1e-9;
     if (px) { bx = 16; by = 16; bi = 1; }
   }
-  tma::TmaP P;
+  tc::TmaP P;
   memset(&P, 0, sizeof(P));
   GemmP g = g0;
   g.K = 9 * C;
@@ -782,14 +643,7 @@ static int gemm_tma_launch_conv(const GemmP& g0, const uint4* Wp, float out_scal
   g.tile_tab = nullptr;
   g.Y = reinterpret_cast<float*>(Yhi);
   g.y_ms = g.M;
-  P.t.g = g;
-  P.t.Wp = Wp;
-  P.t.m_tiles = (g.M + 127) / 128;
-  P.t.k_chunks = g.K / tc::BK;
-  P.t.mt_per_cta = P.t.m_tiles >= 2 ? 2 : 1;
-  P.t.out_scale = out_scale;
-  P.t.out_mode = tma::OUT_PLANAR;
-  P.t.dbg = mm_debug_flags();
+  P.t = tc::tc_params(g, Wp, out_scale, true);
   P.plane_elems = P.pool ? y_plane_pooled : y_plane;
   P.status = status;
   P.ksegs = 1; P.kc_per_seg = P.t.k_chunks;
@@ -804,12 +658,7 @@ static int gemm_tma_launch_conv(const GemmP& g0, const uint4* Wp, float out_scal
   MM_TRY(tma::make_map_4d(&ml, Xhi + x_plane, n_img, H, W, C, bx, box_y, bi));
   if (px) {
     P.t.Wp = Wpx;
-    return gemm_tma_px_launch(P, mh, ml, sms, st);
+    return gemm_tma_px_launch(P, mh, ml, st);
   }
-  const long mgroups = (P.t.m_tiles + P.t.mt_per_cta - 1) / P.t.mt_per_cta;
-  const long total = (long)g.num_tiles * mgroups;
-  const int grid = (int)(total < sms ? total : sms);
-  tma::gemm_tma_kernel<<<grid, tma::T_THREADS, tma::T_SMEM_BYTES, st>>>(P, mh, ml);
-  MM_LAUNCH_CHECK();
-  return 0;
+  return gemm_tma_launch(P, mh, ml, st);
 }

@@ -22,7 +22,7 @@ constexpr int PX_W_SLOT = 8192;                 // one k chunk of the compact we
 constexpr int PX_X_OFF = 3 * PX_W_SLOT;         // 24 KB: three tap slots
 constexpr int PX_X_PLANE = 24576;               // up to 384 box rows x 64 B per plane
 constexpr int PX_STAGE = PX_X_OFF + 2 * PX_X_PLANE;   // 72 KB
-constexpr size_t PX_SMEM_BYTES = (size_t)STAGES * PX_STAGE + 1024 + 256;
+constexpr size_t PX_SMEM_BYTES = tc_smem_bytes(PX_STAGE);
 
 constexpr uint32_t IDESC_N64 = (1u << 4) | ((64u >> 3) << 17) | ((128u >> 4) << 24);
 constexpr uint32_t IDESC_N128 = (1u << 4) | ((128u >> 3) << 17) | ((128u >> 4) << 24);
@@ -46,16 +46,6 @@ gemm_tma_px_kernel(const TmaP P, const __grid_constant__ CUtensorMap map_hi, con
   const GemmP& p = P.t.g;
   extern __shared__ uint8_t smem_raw[];
   __shared__ float s_bias[64];
-  const uint32_t raw = smem_u32(smem_raw);
-  const uint32_t base = (raw + 1023u) & ~1023u;
-  uint8_t* sm = smem_raw + (base - raw);
-  const uint32_t bar0 = base + STAGES * PX_STAGE;
-  auto full_bar = [&](int s) { return bar0 + 8u * s; };
-  auto empty_bar = [&](int s) { return bar0 + 8u * (STAGES + s); };
-  auto tfull_bar = [&](int b) { return bar0 + 8u * (2 * STAGES + b); };
-  auto tempty_bar = [&](int b) { return bar0 + 8u * (2 * STAGES + 2 + b); };
-  uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(sm + STAGES * PX_STAGE + 8 * (2 * STAGES + 4));
-
   const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
   const long total_tiles = p.num_tiles;
   const int cchunks = P.C / BK;                          // conv: channel chunks per tap
@@ -64,34 +54,8 @@ gemm_tma_px_kernel(const TmaP P, const __grid_constant__ CUtensorMap map_hi, con
   const uint32_t xbytes = P.conv ? (uint32_t)(P.bx * (P.by + 2) * 64) : (uint32_t)B_HALF;
 
   if (tid < 64) s_bias[tid] = p.bias ? p.bias[tid] : 0.f;
-  if (tid == 0) {
-    for (int s = 0; s < STAGES; s++) {
-      mbar_init(full_bar(s), GEN27 ? 1 + PX_GEN_WARPS : 1);
-      mbar_init(empty_bar(s), 1);
-    }
-    for (int b = 0; b < 2; b++) {
-      mbar_init(tfull_bar(b), 1);
-      mbar_init(tempty_bar(b), T_EPI_WARPS);
-    }
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-  }
-  if (warp == T_MMA_WARP) {
-    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(tmem_slot)),
-                 "r"(512)
-                 : "memory");
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
-  }
-  tc_fence_before();
-  __syncthreads();
-  tc_fence_after();
-  const uint32_t tmem_base = *tmem_slot;
-
-  auto conv_origin = [&](int nt, int& i0, int& y0, int& x0) {
-    const int tx = nt % P.tiles_x;
-    const int r = nt / P.tiles_x;
-    const int ty = r % P.tiles_y;
-    i0 = (r / P.tiles_y) * P.bi; y0 = ty * P.by; x0 = tx * P.bx;
-  };
+  // full: the loader's expect_tx arrive (+ one arrive per GEN27 producer warp of a group)
+  const TcPipe C = tc_begin<PX_STAGE>(smem_raw, GEN27 ? 1 + PX_GEN_WARPS : 1, T_EPI_WARPS, warp == T_MMA_WARP);
 
   if (warp < T_EPI_WARPS) {
     // =============================== EPILOGUE ===============================
@@ -102,9 +66,9 @@ gemm_tma_px_kernel(const TmaP P, const __grid_constant__ CUtensorMap map_hi, con
     // an int tile index (tile counts are < 2^31) keeps the GEN27 variant, at its 96-register cap, from spilling wcount
     for (int nt = blockIdx.x; nt < total_tiles; nt += gridDim.x, wcount++) {
       int i0 = 0, y0 = 0, x0 = 0;
-      if (P.conv) conv_origin(nt, i0, y0, x0);
-      const int abuf = (int)(wcount & 1);
-      mbar_wait(tfull_bar(abuf), (wcount >> 1) & 1);
+      if (P.conv) conv_origin(P, nt, i0, y0, x0);
+      const int abuf = acc_buf(wcount, 2);
+      mbar_wait(C.tfull_bar(abuf), acc_parity(wcount, 2));
       tc_fence_after();
 #pragma unroll 1
       for (int sub = 0; sub < 2; sub++) {
@@ -124,8 +88,8 @@ gemm_tma_px_kernel(const TmaP P, const __grid_constant__ CUtensorMap map_hi, con
         }
         // accumulator = columns [0, 64) (hi*hi + lo*hi) + columns [64, 128) (hi*lo partial)
         uint32_t v[32], v2[32];
-        tmem_ld32(tmem_base + ((uint32_t)(q * 32) << 16) + (uint32_t)(abuf * 256 + sub * 128 + cb), v);
-        tmem_ld32(tmem_base + ((uint32_t)(q * 32) << 16) + (uint32_t)(abuf * 256 + sub * 128 + 64 + cb), v2);
+        tmem_ld32(C.tmem + ((uint32_t)(q * 32) << 16) + (uint32_t)(abuf * 256 + sub * 128 + cb), v);
+        tmem_ld32(C.tmem + ((uint32_t)(q * 32) << 16) + (uint32_t)(abuf * 256 + sub * 128 + 64 + cb), v2);
 #pragma unroll
         for (int j = 0; j < 32; j++) v[j] = __float_as_uint(__uint_as_float(v[j]) + __uint_as_float(v2[j]));
         if (P.t.dbg & 1) continue;
@@ -161,7 +125,7 @@ gemm_tma_px_kernel(const TmaP P, const __grid_constant__ CUtensorMap map_hi, con
           // 8 KB scratch [plane][pixel][128 B] (16-byte chunk c of pixel p at slot c ^ (p & 7): conflict-free both ways)
           // in an unused tail of the stage buffers; then one warp stores the hi plane, the other the lo plane, every
           // instruction writing 8 complete lines.
-          const uint32_t scr = base + (uint32_t)((q >> 1) * PX_STAGE + PX_X_OFF + (q & 1) * PX_X_PLANE + 16384);
+          const uint32_t scr = C.base + (uint32_t)((q >> 1) * PX_STAGE + PX_X_OFF + (q & 1) * PX_X_PLANE + 16384);
           const uint32_t rowa = scr + (uint32_t)lane * 128u;
 #pragma unroll
           for (int k = 0; k < 4; k++) {
@@ -197,7 +161,7 @@ gemm_tma_px_kernel(const TmaP P, const __grid_constant__ CUtensorMap map_hi, con
       }
       tc_fence_before();
       __syncwarp();
-      if (lane == 0) mbar_arrive(tempty_bar(abuf));
+      if (lane == 0) mbar_arrive(C.tempty_bar(abuf));
     }
     mm_range_flag2(P.status, racc);
   } else if (warp == T_MMA_WARP) {
@@ -205,14 +169,14 @@ gemm_tma_px_kernel(const TmaP P, const __grid_constant__ CUtensorMap map_hi, con
     if (lane == 0) {
       uint32_t it = 0, tcount = 0;
       for (long t = blockIdx.x; t < total_tiles; t += gridDim.x, tcount++) {
-        const int abuf = (int)(tcount & 1);
-        mbar_wait(tempty_bar(abuf), ((tcount >> 1) & 1) ^ 1);
+        const int abuf = acc_buf(tcount, 2);
+        mbar_wait(C.tempty_bar(abuf), acc_parity(tcount, 2) ^ 1);
         tc_fence_after();
         for (int si = 0; si < nstage; si++, it++) {
-          const int s = it % STAGES;
-          mbar_wait(full_bar(s), (it / STAGES) & 1);
+          const int s = ring_stage(it);
+          mbar_wait(C.full_bar(s), ring_parity(it));
           tc_fence_after();
-          const uint32_t sw = base + s * PX_STAGE, sx = sw + PX_X_OFF;
+          const uint32_t sw = C.base + s * PX_STAGE, sx = sw + PX_X_OFF;
           if (!(P.t.dbg & 8)) {
             for (int ky = 0; ky < ntap; ky++) {
               const uint32_t xo = sx + (uint32_t)(ky * P.bx * 64), wo = sw + (uint32_t)(ky * PX_W_SLOT);
@@ -223,15 +187,15 @@ gemm_tma_px_kernel(const TmaP P, const __grid_constant__ CUtensorMap map_hi, con
                   const uint64_t x_hi = smem_desc_sw64(xo + sub * (128 * 64) + ks * 32);
                   const uint64_t x_lo = smem_desc_sw64(xo + PX_X_PLANE + sub * (128 * 64) + ks * 32);
                   const uint64_t w_hl = smem_desc(wo + ks * 2 * PX_WC_LBO, PX_WC_LBO, SBO);   // rows 0-63 W_hi, 64-127 W_lo
-                  const uint32_t d = tmem_base + (uint32_t)(abuf * 256 + sub * 128);
+                  const uint32_t d = C.tmem + (uint32_t)(abuf * 256 + sub * 128);
                   umma_f16(d, x_hi, w_hl, IDESC_N128, (si | ky | ks) ? 1u : 0u);
                   umma_f16(d, x_lo, w_hl, IDESC_N64, 1u);
                 }
               }
             }
           }
-          umma_commit(empty_bar(s));
-          if (si == nstage - 1) umma_commit(tfull_bar(abuf));
+          umma_commit(C.empty_bar(s));
+          if (si == nstage - 1) umma_commit(C.tfull_bar(abuf));
         }
       }
     }
@@ -250,17 +214,17 @@ gemm_tma_px_kernel(const TmaP P, const __grid_constant__ CUtensorMap map_hi, con
     float amax = 0.f;
     uint32_t it = (uint32_t)grp;
     for (long t = blockIdx.x + (long)grp * gridDim.x; t < total_tiles; t += 2L * gridDim.x, it += 2) {
-      const int s = it % STAGES;
+      const int s = ring_stage(it);
       const long row0 = t * BN;
       const long img = row0 / hw;
       const int r0 = (int)(row0 - img * hw);
       const float* src = P.gen_src + img * 3 * hw;
-      mbar_wait(empty_bar(s), ((it / STAGES) & 1) ^ 1);
-      float* stg = reinterpret_cast<float*>(sm + s * PX_STAGE + PX_W_SLOT);
+      mbar_wait(C.empty_bar(s), ring_parity(it) ^ 1);
+      float* stg = reinterpret_cast<float*>(C.sm + s * PX_STAGE + PX_W_SLOT);
       const int lin0 = r0 - W - 1;
       if (P.t.dbg & 4) {                         // profiling: no operand generation (results wrong)
         __syncwarp();
-        if (lane == 0) mbar_arrive(full_bar(s));
+        if (lane == 0) mbar_arrive(C.full_bar(s));
         continue;
       }
 #pragma unroll 1
@@ -277,7 +241,7 @@ gemm_tma_px_kernel(const TmaP P, const __grid_constant__ CUtensorMap map_hi, con
           if (i0 + u * 128 < 3 * span) stg[i0 + u * 128] = q[u];
       }
       asm volatile("bar.sync %0, 128;" ::"r"(1 + grp) : "memory");
-      const uint32_t sx = base + s * PX_STAGE + PX_X_OFF;
+      const uint32_t sx = C.base + s * PX_STAGE + PX_X_OFF;
 #pragma unroll
       for (int j = 0; j < 2; j++) {
         const int rr = j * 128 + pt;
@@ -314,7 +278,7 @@ gemm_tma_px_kernel(const TmaP P, const __grid_constant__ CUtensorMap map_hi, con
       }
       asm volatile("fence.proxy.async.shared::cta;" ::: "memory");   // generic-proxy writes -> visible to the MMA's async proxy
       __syncwarp();
-      if (lane == 0) mbar_arrive(full_bar(s));
+      if (lane == 0) mbar_arrive(C.full_bar(s));
     }
     mm_range_flag(P.status, amax);
   } else {
@@ -324,24 +288,24 @@ gemm_tma_px_kernel(const TmaP P, const __grid_constant__ CUtensorMap map_hi, con
       for (long t = blockIdx.x; t < total_tiles; t += gridDim.x) {
         const int nt = (int)t;
         int i0 = 0, y0 = 0, x0 = 0;
-        if (P.conv) conv_origin(nt, i0, y0, x0);
+        if (P.conv) conv_origin(P, nt, i0, y0, x0);
         for (int si = 0; si < nstage; si++, it++) {
-          const int s = it % STAGES;
-          mbar_wait(empty_bar(s), ((it / STAGES) & 1) ^ 1);
-          mbar_expect_tx(full_bar(s), (uint32_t)ntap * PX_W_SLOT + (GEN27 ? 0u : 2u * xbytes));
-          const uint32_t sw = base + s * PX_STAGE, sx = sw + PX_X_OFF;
+          const int s = ring_stage(it);
+          mbar_wait(C.empty_bar(s), ring_parity(it) ^ 1);
+          mbar_expect_tx(C.full_bar(s), (uint32_t)ntap * PX_W_SLOT + (GEN27 ? 0u : 2u * xbytes));
+          const uint32_t sw = C.base + s * PX_STAGE, sx = sw + PX_X_OFF;
           const int kx = P.conv ? si / cchunks : 0, cc = P.conv ? si - kx * cchunks : 0;
           for (int ky = 0; ky < ntap; ky++) {
             // weights pre-packed for N = 64 (weights.py::pack_px): one 8 KB copy per k chunk
             const int kc = P.conv ? (ky * 3 + kx) * cchunks + cc : si;
-            bulk_g2s(sw + ky * PX_W_SLOT, reinterpret_cast<const uint8_t*>(P.t.Wp) + (size_t)kc * PX_W_SLOT, PX_W_SLOT, full_bar(s));
+            bulk_g2s(sw + ky * PX_W_SLOT, reinterpret_cast<const uint8_t*>(P.t.Wp) + (size_t)kc * PX_W_SLOT, PX_W_SLOT, C.full_bar(s));
           }
           if (P.conv) {
-            tma_load_4d(sx, &map_hi, cc * BK, x0 + kx - 1, y0 - 1, i0, full_bar(s));
-            tma_load_4d(sx + PX_X_PLANE, &map_lo, cc * BK, x0 + kx - 1, y0 - 1, i0, full_bar(s));
+            tma_load_4d(sx, &map_hi, cc * BK, x0 + kx - 1, y0 - 1, i0, C.full_bar(s));
+            tma_load_4d(sx + PX_X_PLANE, &map_lo, cc * BK, x0 + kx - 1, y0 - 1, i0, C.full_bar(s));
           } else if (!GEN27) {
-            tma_load_2d(sx, &map_hi, si * BK, nt * BN, full_bar(s));
-            tma_load_2d(sx + PX_X_PLANE, &map_lo, si * BK, nt * BN, full_bar(s));
+            tma_load_2d(sx, &map_hi, si * BK, nt * BN, C.full_bar(s));
+            tma_load_2d(sx + PX_X_PLANE, &map_lo, si * BK, nt * BN, C.full_bar(s));
           }
         }
       }
@@ -349,11 +313,7 @@ gemm_tma_px_kernel(const TmaP P, const __grid_constant__ CUtensorMap map_hi, con
     __syncwarp();
   }
 
-  tc_fence_before();
-  __syncthreads();
-  if (warp == T_MMA_WARP) {
-    asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(512) : "memory");
-  }
+  tc_end(*C.tmem_slot(), warp == T_MMA_WARP);
 }
 
 }  // namespace tma

@@ -1,6 +1,7 @@
 // GroupNorm statistics -> per-(group, channel) affine, and a few small shared kernels.
+// Compiled in engines.cu only: the launchers below have external linkage (see engines.cuh).
 #pragma once
-#include "common.cuh"
+#include "engines.cuh"
 
 // stats[G][C][2] (sum, sumsq over the group's columns, fp64) -> sc/sh[G][C] so that
 //   GroupNorm(x)[c] = x*sc + sh,   sc = gamma[c]*rstd,  sh = beta[c] - mean*sc.
@@ -41,8 +42,8 @@ static __global__ void __launch_bounds__(256) stats_reduce_kernel(const double2*
   }
 }
 
-static inline int stats_reduce(const double2* part, int M, int G, int tpg, const int* gstart, double* stats,
-                               cudaStream_t st, int mult = 1) {
+int stats_reduce(const double2* part, int M, int G, int tpg, const int* gstart, double* stats, cudaStream_t st,
+                 int mult) {
   dim3 grid(mm_cdiv(M, 32), G), block(32, 8);
   stats_reduce_kernel<<<grid, block, 0, st>>>(part, M, G, tpg, gstart, mult, stats);
   MM_LAUNCH_CHECK();
@@ -76,9 +77,8 @@ static __global__ void gn_finalize_kernel(const double* __restrict__ stats, cons
   if (status && sqrt(n) * fabs((double)gamma[c]) + fabs((double)beta[c]) >= 65504.0) atomicOr(status, 1);
 }
 
-static inline int gn_finalize(const double* stats, const float* gamma, const float* beta, const int* cnt,
-                              int uniform, int G, int C, int cpg, float* sc, float* sh,
-                              cudaStream_t st, int stats_ld = 0, int c_off = 0, int* status = nullptr) {
+int gn_finalize(const double* stats, const float* gamma, const float* beta, const int* cnt, int uniform, int G, int C,
+                int cpg, float* sc, float* sh, cudaStream_t st, int stats_ld, int c_off, int* status) {
   gn_finalize_kernel<<<mm_cdiv((long)G * C, 256), 256, 0, st>>>(
       stats, gamma, beta, cnt, uniform, G, C, cpg, stats_ld ? stats_ld : C, c_off, sc, sh, status);
   MM_LAUNCH_CHECK();

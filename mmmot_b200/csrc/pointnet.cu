@@ -8,9 +8,7 @@
 // Per-detection pooling is a MEAN (SURVEY F5).  One frame-pair = one GroupNorm domain.
 #include <vector>
 
-#include "norm_ops.cuh"
-#include "gemm_gen.cuh"
-#include "tc_ops.cuh"
+#include "engines.cuh"
 
 namespace {
 
@@ -124,17 +122,8 @@ __global__ void pointnet_out_kernel(const float* __restrict__ O, const float* __
   feats[(((long)pair * 3 + 1) * 512 + c) * L + l] = v;
 }
 
-// out[c][d] = segsum[d][c] * 2^-32 / (points of detection d)   (fixed-point sums of the fused segment-sum epilogue)
-__global__ void segsum_mean_kernel(const unsigned long long* __restrict__ segsum, const int* __restrict__ split,
-                                   int C, int ndet, float* __restrict__ out) {
-  long idx = (long)blockIdx.x * blockDim.x + threadIdx.x;
-  if (idx >= (long)C * ndet) return;
-  const int d = (int)(idx / C), c = (int)(idx - (long)d * C);
-  const int cnt = split[d + 1] - split[d];
-  out[(long)c * ndet + d] = cnt > 0 ? (float)((double)segsum[idx] * (1.0 / 4294967296.0) / (double)cnt) : 0.f;
-}
-
-// channels-last variant: out[d][C] (the layout the tensor-core per-detection contractions read as rows)
+// out[d][C] = segsum[d][C] * 2^-32 / (points of detection d): the fixed-point sums of the fused segment-sum epilogue, in
+// the layout the tensor-core per-detection contractions read as rows
 __global__ void segsum_mean_cl_kernel(const unsigned long long* __restrict__ segsum, const int* __restrict__ split,
                                       int C, int ndet, float* __restrict__ out) {
   long idx = (long)blockIdx.x * blockDim.x + threadIdx.x;
@@ -289,8 +278,7 @@ static int pointnet_impl(const mmmot_weights* wts, const float* points, const in
   point_segment_kernel<<<mm_cdiv(P, 256), 256, 0, st>>>(det_split, ndet, P, w.seg);
   MM_LAUNCH_CHECK();
   if (use_tc) {
-    tma::seg_chunk_tab_kernel<<<mm_cdiv(n_tiles * 2, 128), 128, 0, st>>>(w.tiles, (int)n_tiles, w.seg, w.ctab);
-    MM_LAUNCH_CHECK();
+    MM_TRY(seg_chunk_tab(w.tiles, (int)n_tiles, w.seg, w.ctab, st));
   }
 
   const int cin[5] = {3, 64, 64, 64, 128}, cout[5] = {64, 64, 64, 128, 1024};
@@ -324,7 +312,7 @@ static int pointnet_impl(const mmmot_weights* wts, const float* points, const in
           // (gemm_gen.cuh) straight from its fp32 output: no normalised copy is written
           MM_TRY((gemm_gen_launch<gen::GEN_NORM>(p, wp, wps, ybuf[i - 1], cin[i], w.sc, w.sh, 0, 0, 0, st)));
         } else {                                                // FP16 hi/lo planes [2][P][cin] via TMA
-          MM_TRY(gemm_tma_launch_mat(p, wp, wps, i == 1 ? w.x1p : w.xp, P * cin[i], P, cin[i], tc::OUT_CL, 0, st));
+          MM_TRY(gemm_tma_launch_mat(p, wp, wps, i == 1 ? w.x1p : w.xp, P * cin[i], P, cin[i], st));
         }
         if (timed) mm_timing_end(st);
       }
@@ -348,7 +336,7 @@ static int pointnet_impl(const mmmot_weights* wts, const float* points, const in
         p.Y = nullptr; p.part = nullptr;
         p.sc = w.sc; p.sh = w.sh; p.seg = w.seg;
         if (timed) mm_timing_begin(st, MM_T_PN_L5B, 2.0 * cout[i] * cin[i] * cols, 4.0 * cin[i] * cols);
-        MM_TRY(gemm_tma_launch_mat(p, wp, wps, w.xp, P * cin[i], P, cin[i], tc::OUT_CL, 0, st, w.segsum, nullptr, w.ctab));
+        MM_TRY(gemm_tma_launch_mat(p, wp, wps, w.xp, P * cin[i], P, cin[i], st, w.segsum, w.ctab));
         if (timed) mm_timing_end(st);
         segsum_mean_cl_kernel<<<mm_cdiv(1024L * ndet, 256), 256, 0, st>>>(w.segsum, det_split, 1024, ndet, w.gmean);
         MM_LAUNCH_CHECK();
@@ -375,7 +363,7 @@ static int pointnet_impl(const mmmot_weights* wts, const float* points, const in
       const uint4* whp = (const uint4*)wts->w[MMMOT_W_PN_WHAP];
       const float whs = wts->tc_scale[MMMOT_W_PN_WHAP];
       if (timed) mm_timing_begin(st, MM_T_PN_HEADA, 2.0 * 512 * 64 * (double)P, 4.0 * 64 * (double)P);
-      MM_TRY(gemm_tma_launch_mat(p, whp, whs, w.x1p, P * 64, P, 64, tc::OUT_CL, 0, st, nullptr, nullptr, w.ctab));
+      MM_TRY(gemm_tma_launch_mat(p, whp, whs, w.x1p, P * 64, P, 64, st, nullptr, w.ctab));
       if (timed) mm_timing_end(st);
       MM_TRY(stats_reduce(w.part, 512, pairs, 0, w.gstart, w.stats, st, 2));
       MM_TRY(gn_finalize(w.stats, wts->w[MMMOT_W_PN_GHW], wts->w[MMMOT_W_PN_GHB], w.cnt, 0, pairs, 512, 1, w.sc, w.sh, st));
@@ -383,7 +371,7 @@ static int pointnet_impl(const mmmot_weights* wts, const float* points, const in
       MM_CUDA(cudaMemsetAsync(w.segsum, 0, (size_t)ndet * 512 * sizeof(unsigned long long), st));
       p.part = nullptr; p.sc = w.sc; p.sh = w.sh;
       if (timed) mm_timing_begin(st, MM_T_PN_HEADB, 2.0 * 512 * 64 * (double)P, 4.0 * 64 * (double)P);
-      MM_TRY(gemm_tma_launch_mat(p, whp, whs, w.x1p, P * 64, P, 64, tc::OUT_CL, 0, st, w.segsum, nullptr, w.ctab));
+      MM_TRY(gemm_tma_launch_mat(p, whp, whs, w.x1p, P * 64, P, 64, st, w.segsum, w.ctab));
       if (timed) mm_timing_end(st);
       segsum_mean_cl_kernel<<<mm_cdiv(512L * ndet, 256), 256, 0, st>>>(w.segsum, det_split, 512, ndet, w.hmean);
       MM_LAUNCH_CHECK();

@@ -1,17 +1,9 @@
 // Small kernels of the tensor-core (channels-last) pipeline: activations between tcgen05 contractions
 // are stored [row][channel], fp32 before the GroupNorm statistics are known and packed FP16 (hi|lo)
 // after normalisation.
+// Compiled in engines.cu only: the launchers below have external linkage (see engines.cuh).
 #pragma once
-#include "gemm_tma.cuh"
-
-__device__ __forceinline__ void split4_store(float4 x, __half* hi, __half* lo, int* status) {
-  mm_range_flag(status, fmaxf(fmaxf(fabsf(x.x), fabsf(x.y)), fmaxf(fabsf(x.z), fabsf(x.w))));
-  __half h[4], l[4];
-  tma::split_f16(x.x, h[0], l[0]); tma::split_f16(x.y, h[1], l[1]);
-  tma::split_f16(x.z, h[2], l[2]); tma::split_f16(x.w, h[3], l[3]);
-  *reinterpret_cast<uint2*>(hi) = *reinterpret_cast<uint2*>(h);
-  *reinterpret_cast<uint2*>(lo) = *reinterpret_cast<uint2*>(l);
-}
+#include "engines.cuh"
 
 // out planes [2][rows][C] (hi, lo) = split(relu(in[row][c]*sc[g][c] + sh[g][c])),
 // g = seg ? seg[row] / L : row / rows_per_group.  GroupNorm + ReLU of the producer layer applied once per
@@ -34,8 +26,8 @@ static __global__ void norm_split_kernel(const float* __restrict__ in, long ldi,
   split4_store(y, out + row * C + c, out + rows * C + row * C + c, status);
 }
 
-static inline int norm_split(const float* in, long ldi, const float* sc, const float* sh, int C, long rows,
-                             int rows_per_group, const int* seg, int L, __half* out, cudaStream_t st, int* status) {
+int norm_split(const float* in, long ldi, const float* sc, const float* sh, int C, long rows, int rows_per_group,
+               const int* seg, int L, __half* out, cudaStream_t st, int* status) {
   norm_split_kernel<<<mm_cdiv(rows * (C / 4), 256), 256, 0, st>>>(in, ldi, sc, sh, C, rows, rows_per_group, seg, L, out,
                                                                  status);
   MM_LAUNCH_CHECK();
@@ -60,7 +52,7 @@ static __global__ void transpose_kernel(const float* __restrict__ src, float* __
     if (r < rows && c < cols) d[(long)c * rows + r] = tile[threadIdx.x][i];
   }
 }
-static inline int transpose_f32(const float* src, float* dst, int rows, int cols, int groups, cudaStream_t st) {
+int transpose_f32(const float* src, float* dst, int rows, int cols, int groups, cudaStream_t st) {
   dim3 grid(mm_cdiv(cols, 32), mm_cdiv(rows, 32), groups), block(32, 8);
   transpose_kernel<<<grid, block, 0, st>>>(src, dst, rows, cols, groups);
   MM_LAUNCH_CHECK();
@@ -75,4 +67,9 @@ static __global__ void feats_range_kernel(const float* __restrict__ f, long n, f
   for (long i = (long)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (long)gridDim.x * blockDim.x)
     amax = fmaxf(amax, fabsf(f[i]));
   if (status && !(amax < limit)) atomicOr(status, 1);
+}
+int feats_range_check(const float* f, long n, float limit, int* status, cudaStream_t st) {
+  feats_range_kernel<<<148, 256, 0, st>>>(f, n, limit, status);
+  MM_LAUNCH_CHECK();
+  return 0;
 }

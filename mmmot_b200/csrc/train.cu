@@ -6,8 +6,7 @@
 // These variants run on the FP32 FFMA engine (gemm_simt.cuh): convolution with the UNFOLDED weights + per-tile
 // (sum, sumsq) partials -> fixed-order reduction -> per-channel affine -> normalise + ReLU in place.  The batch
 // statistics are returned so that the host can update the module's running averages like torch does.
-#include "gemm_simt.cuh"
-#include "norm_ops.cuh"
+#include "engines.cuh"
 
 namespace {
 

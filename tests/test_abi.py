@@ -1,9 +1,12 @@
 """CPU: the C-ABI library loads and exports every symbol include/mmmot_b200.h declares; the Python
 mirror of the enums/weight ids matches the header; host-side logic (schema, weight packing,
 config surface, error behaviour without a GPU)."""
+import collections
 import ctypes
 import os
 import re
+import shutil
+import subprocess
 
 import pytest
 import torch
@@ -63,6 +66,16 @@ def test_set_debug_accepts_only_the_profiling_bits(lib_built):
             assert lib.mmmot_set_debug(flags) == -1, flags
     finally:
         lib.mmmot_set_debug(0)
+
+
+@pytest.mark.skipif(shutil.which("cuobjdump") is None, reason="needs cuobjdump")
+def test_every_kernel_is_compiled_once(lib_built):
+    """The kernels are compiled in one translation unit (engines.cu), so the library holds one body per kernel."""
+    sass = subprocess.run(["cuobjdump", "-sass", _lib.LIB_PATH], capture_output=True, text=True, check=True).stdout
+    names = re.findall(r"Function : (\S+)", sass)
+    assert names
+    dups = sorted(n for n, c in collections.Counter(names).items() if c > 1)
+    assert not dups, dups
 
 
 @pytest.mark.parametrize("fusion,nkeys,numel",[("C", 263, 21218212), ("A", 255, None), ("B", 259, None)])
